@@ -56,6 +56,7 @@ def load() -> C.CDLL:
     lib.bis_host_bench_setup_ms.restype = C.c_double
     lib.bis_host_bench_history.argtypes = [C.c_void_p, C.c_void_p, C.c_int]
     lib.bis_host_bench_run.argtypes = [C.c_void_p, C.c_int, C.c_void_p]
+    lib.bis_host_bench_copy_x.argtypes = [C.c_void_p, C.c_void_p]
     _lib = lib
     return lib
 
@@ -255,6 +256,11 @@ class BenchSession:
             raise capi.BisError(_err())
         return {"device_ms": out[0], "wall_ms": out[1], "launches": int(out[2]), "res_last": out[3],
                 "res0": out[4]}
+
+    def copy_x(self, x_dev: int):
+        """Enqueue a copy of the current iterate of a CG session into the device vector x_dev (local rows)."""
+        if self.lib.bis_host_bench_copy_x(self.h, x_dev) != 0:
+            raise capi.BisError(_err())
 
     def close(self):
         if self.h:

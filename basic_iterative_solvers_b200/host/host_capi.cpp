@@ -399,4 +399,19 @@ int bis_host_bench_run(void *h, int steps, double *out) {
     }
 }
 
+// Enqueues a copy of the current iterate of a CG session (x after the last step run: what save_x_star() would
+// hand back) into the device vector x_dev of the session's local rows.  The session's state is not touched.
+int bis_host_bench_copy_x(void *h, double *x_dev) {
+    auto *s = static_cast<BenchSession *>(h);
+    try {
+        auto *cg = dynamic_cast<ConjugateGradientSolver *>(s->solver.get());
+        if (!cg) bis_fatal("bench: copy_x needs a prepared CG session");
+        copy_vector(s->dev, x_dev, cg->x_old, cg->N);
+        return 0;
+    } catch (const std::exception &e) {
+        g_host_err = e.what();
+        return 1;
+    }
+}
+
 } // extern "C"

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- BASELINE.json's metric: PCG time/iteration and SpMV HBM GB/s vs roofline on HPCG-512.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--grid 512]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--grid 512] [--dump-outputs DIR]
 
 A "step" is ONE iteration of the solver harness loop (solver_harness.hpp:17-50 of the
 reference: iterate, residual-norm sample read back by the host, pointer exchange) of
@@ -16,6 +16,11 @@ x_star downloaded, residual norm read back every iteration); `roofline` is the S
 (oracle/_ref) timed on the host cores on a bounded sample.
 
 `--impl reference` times the reference's own CPU implementation of the same path (rank 0 only).
+
+`--dump-outputs DIR` (one GPU) writes what the timed loop computed in its last step, for comparing two builds output
+for output (the inputs are the same on every run): DIR/residual_norms.npy, ||r_0|| .. ||r_(W+K)|| of the session, and
+the iterate x_(W+K) at a fixed seeded sample of DUMP_X_SAMPLE rows, DIR/x_sample.npy (values) and
+DIR/x_sample_rows.npy (row numbers); float64, 16 MB in all.
 """
 from __future__ import annotations
 
@@ -196,6 +201,7 @@ def pick_cpu_sample(n_target: int) -> int:
 
 PARITY_GOLDEN = os.path.join(ROOT, "tests", "golden", "bench_parity.json")
 PARITY_LEN = 25
+DUMP_X_SAMPLE = 1 << 20
 
 
 def parity_block(histories: dict, n: int, world: int, write_to: str | None):
@@ -255,12 +261,21 @@ def main():
     ap.add_argument("--write-parity-golden", default=None, metavar="PATH",
                     help="one GPU: write the parity golden (merged with the committed one) to PATH")
     ap.add_argument("--option", action="append", default=[], metavar="KEY=INT", help="bis_context_set_option")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="one GPU: write what the timed loop computed in its last step to DIR/<name>.npy")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if args.warmup < 3:
         args.warmup = 3
+    # one solver session runs at most MAX_ITERS = 1000 iterations: the warm-up, the timed steps and the initial residual
+    if args.warmup > 997:
+        ap.error("--warmup must be at most 997")
+    if args.steps < 1 or args.warmup + args.steps + 1 >= 1000:
+        ap.error(f"--steps must be in [1, {998 - args.warmup}] with --warmup {args.warmup}")
+    if args.dump_outputs and (world > 1 or args.impl != "ours"):
+        ap.error("--dump-outputs needs one GPU and --impl ours")
     n = args.n
     nz = n * world if args.weak else n
     n_rows_g, nnz_g = n * n * nz, (3 * n - 2) ** 2 * (3 * nz - 2)
@@ -386,6 +401,11 @@ def main():
     t_clk = time.time()
     r = sess.run(K)
     barrier()
+    if args.dump_outputs:
+        # the iterate of the last timed step, copied on the device now (the loop runs on below) and read back later
+        x_last = ctx.alloc(n_local)
+        sess.copy_x(x_last)
+        dump = {"residual_norms": sess.history(W + K + 1)}
     waits = ctx.dist_wait_read(reset=True) if world > 1 else None
     # a short timed region (tens of ms at 8 GPUs) gives the sampler nothing to see: keep the same
     # iteration loop running, untimed and unreported, until the sampler has watched ~0.6 s of it
@@ -396,6 +416,18 @@ def main():
     barrier()
     clk = clocks.stop()
     clk["window"] = f"the {K} timed iterations + {extra} further iterations of the same loop (untimed)"
+    if args.dump_outputs:
+        x = ctx.download(x_last, n_local)
+        ctx.free(x_last)
+        rows = np.arange(n_local)
+        if n_local > DUMP_X_SAMPLE:
+            rows = np.sort(np.random.default_rng(0).choice(n_local, DUMP_X_SAMPLE, replace=False))
+        dump["x_sample"] = x[rows]
+        dump["x_sample_rows"] = rows.astype(np.float64)
+        del x
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for fname, a in dump.items():
+            np.save(os.path.join(args.dump_outputs, fname + ".npy"), a)
     dev_ms = max_over_ranks(r["device_ms"])
     launches = r["launches"]
     ms_iter = dev_ms / K

@@ -159,6 +159,54 @@ def scale_fixtures():
     np.savez_compressed(os.path.join(OUT, "anderson_dd_12_10_8_scale.npz"), **d)
 
 
+RANDOM_SOLVES = [("cg", "sgs"), ("bi", "ilu0"), ("gm", "ilu0"), ("sgs", "none")]
+
+
+def random_system(n=300, seed=3):
+    """Symmetric, strictly diagonally dominant matrix with a random sparsity pattern (3 % fill), and a vector x."""
+    rng = np.random.default_rng(seed)
+    dense = (rng.random((n, n)) < 0.03) * rng.uniform(-1, 1, (n, n))
+    dense = dense + dense.T
+    np.fill_diagonal(dense, np.abs(dense).sum(axis=1) + 1.0)
+    rows, cols = np.nonzero(dense)
+    rp = np.zeros(n + 1, np.int32)
+    np.add.at(rp, rows + 1, 1)
+    rp = np.cumsum(rp).astype(np.int32)
+    return rp, cols.astype(np.int32), dense[rows, cols], rng.uniform(-1, 1, n)
+
+
+def random_fixture():
+    """random300.npz: ILU(0) factors, SGS and ILU(0) preconditioner outputs and four whole solves on random_system().
+    Written from the compiled reference when oracle/_ref is built, otherwise from the oracle (oracle/port, which
+    matches the reference bit for bit on the fixtures above); `source` records which.
+
+        python tests/golden/make_golden.py random300
+    """
+    from oracle import port
+    ref = refshim.available()
+    if ref:
+        refshim.load().ref_omp_set_threads(1)
+    impl = refshim if ref else port
+    rp, col, val, x = random_system()
+    d = {"source": np.array(["reference" if ref else "oracle"]), "rp": rp, "col": col, "val": val, "x": x}
+    ilu = impl.factor(rp, col, val, "ilu0")
+    for k in ("l_rp", "l_col", "l_val", "u_rp", "u_col", "u_val", "L_D", "U_D"):
+        d["ilu0__" + k] = getattr(ilu, k)
+    d["precond__ilu0"] = impl.apply_preconditioner("ilu0", ilu, x)
+    d["precond__sgs"] = impl.apply_preconditioner("sgs", impl.factor(rp, col, val, "sgs"), x)
+    for method, pre in RANDOM_SOLVES:
+        r = refshim.solve(rp, col, val, method, pre, threads=1) if ref else port.solve(rp, col, val, method, pre)
+        d[f"{method}__{pre}__history"] = r.history
+        d[f"{method}__{pre}__meta"] = np.array([r.iter_count, int(r.converged), r.restarts], np.int64)
+        print(f"  {method}__{pre}: its={r.iter_count} conv={int(r.converged)} r0={r.history[0]:.6e}")
+    np.savez_compressed(os.path.join(OUT, "random300.npz"), **d)
+    print(f"random300.npz written from the {d['source'][0]}")
+
+
+if __name__ == "__main__" and len(sys.argv) > 1 and sys.argv[1] == "random300":
+    random_fixture()
+    raise SystemExit(0)
+
 if __name__ == "__main__" and not (len(sys.argv) > 1 and sys.argv[1] == "twostage"):
     if len(sys.argv) > 1 and sys.argv[1] == "scale":
         scale_fixtures()

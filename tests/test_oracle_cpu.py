@@ -183,25 +183,52 @@ def test_golden_solves(name):
         check_against_fixture(got, g, key)
 
 
-# ---- (3) live against the compiled reference (build container only) -------------------------
-needs_ref = pytest.mark.skipif(not refshim.available(), reason="oracle/_ref not built")
+# ---- (3) a random sparsity pattern: stored fixture, and live against the compiled reference where it is built ----
+def _dense(rp, col, val, n):
+    d = np.zeros((n, n))
+    d[np.repeat(np.arange(n), np.diff(rp)), col] = val
+    return d
 
 
-@needs_ref
 def test_live_reference_random_matrix():
-    rng = np.random.default_rng(3)
-    n = 300
-    dense = (rng.random((n, n)) < 0.03) * rng.uniform(-1, 1, (n, n))
-    dense = dense + dense.T
-    np.fill_diagonal(dense, np.abs(dense).sum(axis=1) + 1.0)
-    rows, cols = np.nonzero(dense)
-    rp = np.zeros(n + 1, np.int32)
-    np.add.at(rp, rows + 1, 1)
-    rp = np.cumsum(rp).astype(np.int32)
-    col, val = cols.astype(np.int32), dense[rows, cols]
+    """Symmetric diagonally dominant 300 x 300 matrix with a random pattern (tests/golden/make_golden.py random300):
+    the oracle against the stored ILU(0) factors, preconditioner outputs and solves (bit-exact / 1e-10 * ||r0||,
+    same counts); the stored values against their defining equations in dense arithmetic; and, where oracle/_ref is
+    built, the oracle against the compiled reference live."""
+    g = golden("random300")
+    rp, col, val, x = g["rp"], g["col"], g["val"], g["x"]
+    n = rp.size - 1
+    fp = port.factor(rp, col, val, "ilu0")
+    for k in ("l_rp", "l_col", "l_val", "u_rp", "u_col", "u_val", "L_D", "U_D"):
+        assert np.array_equal(getattr(fp, k), g["ilu0__" + k]), k
+    assert np.array_equal(port.apply_preconditioner("ilu0", fp, x), g["precond__ilu0"])
+    assert np.array_equal(port.apply_preconditioner("sgs", port.factor(rp, col, val, "sgs"), x), g["precond__sgs"])
+    for key in sorted(k[:-len("__history")] for k in g.files if k.endswith("__history")):
+        method, pre = key.split("__")
+        r, want = port.solve(rp, col, val, method, pre), g[key + "__history"]
+        its, conv, restarts = (int(v) for v in g[key + "__meta"])
+        assert (r.iter_count, r.converged, r.restarts) == (its, bool(conv), restarts), key
+        assert r.history.size == want.size and np.max(np.abs(r.history - want)) <= HIST_TOL * want[0], key
+
+    # the stored values in dense arithmetic: ILU(0) reproduces A on its pattern, the preconditioner outputs solve
+    # their systems, every history starts at ||b - A x0|| (b = 1, x0 = 0.1) and the solves converged
+    A = _dense(rp, col, val, n)
+    L = np.eye(n) + _dense(g["ilu0__l_rp"], g["ilu0__l_col"], g["ilu0__l_val"], n)
+    U = np.diag(g["ilu0__U_D"]) + _dense(g["ilu0__u_rp"], g["ilu0__u_col"], g["ilu0__u_val"], n)
+    assert np.array_equal(g["ilu0__L_D"], np.ones(n))
+    assert np.max(np.abs((L @ U - A)[A != 0])) <= 1e-13 * np.max(np.abs(A))
+    assert np.linalg.norm(L @ U @ g["precond__ilu0"] - x) <= 1e-13 * np.linalg.norm(x)
+    M = np.tril(A) @ np.diag(1.0 / np.diag(A)) @ np.triu(A)             # (D + L) D^-1 (D + U)
+    assert np.linalg.norm(M @ g["precond__sgs"] - x) <= 1e-13 * np.linalg.norm(x)
+    r0 = np.linalg.norm(np.ones(n) - A @ np.full(n, 0.1))
+    for key in (k[:-len("__history")] for k in g.files if k.endswith("__history")):
+        h = g[key + "__history"]
+        assert abs(h[0] - r0) <= 1e-13 * r0 and g[key + "__meta"][1] == 1 and h[-1] < 1e-14 * h[0], key
+
+    if not refshim.available():
+        return
     refshim.load().ref_omp_set_threads(1)
-    x = rng.uniform(-1, 1, n)
-    fr, fp = refshim.factor(rp, col, val, "ilu0"), port.factor(rp, col, val, "ilu0")
+    fr = refshim.factor(rp, col, val, "ilu0")
     for k in ("l_val", "u_val", "L_D", "U_D"):
         assert np.array_equal(getattr(fr, k), getattr(fp, k)), k
     for pre in ("sgs", "ilu0"):

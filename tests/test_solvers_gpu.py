@@ -159,6 +159,28 @@ def test_device_generated_matrix_equals_uploaded(ctx):
         assert a.iter_count == b.iter_count and np.array_equal(a.history, b.history)
 
 
+def test_bench_session_iterate_copy_matches_solve(ctx):
+    """The iterate a CG bench session copies out after its warm-up and timed steps (bench.py --dump-outputs) is the
+    x_star of a solve stopped after as many iterations, and the session's residual norms are that solve's."""
+    rp, col, val = matgen.hpcg(16)
+    n = rp.size - 1
+    want = host.solve(ctx, "cg", "j", crs=(rp, col, val), max_iters=8)
+    sess = host.BenchSession(ctx, "HPCG-16", "cg", "j")
+    try:
+        sess.prepare(3)
+        sess.run(5)
+        x = ctx.alloc(n)
+        sess.copy_x(x)
+        got = ctx.download(x, n)
+        ctx.free(x)
+        hist = sess.history(16)
+    finally:
+        sess.close()
+    assert hist.size == want.history.size == 9
+    assert np.max(np.abs(hist - want.history)) <= HIST_TOL * want.history[0]
+    assert np.max(np.abs(got - want.x_star)) <= 1e-12 * np.max(np.abs(want.x_star))
+
+
 def test_run_to_run_determinism(ctx):
     rp, col, val = matgen.hpcg(20)
     for method, pre in (("cg", "sgs"), ("gm", "ilu0"), ("bi", "j")):
