@@ -117,6 +117,12 @@ _SIGS = {
     "bis_mgs_step": ([c_ctx, i64, c_dev, c_dev, c_dev, cint, cint], cint),
     "bis_scale_inv_norm": ([c_ctx, i64, c_dev, c_dev, cint], cint),
     "bis_gmres_update_x": ([c_ctx, i64, cint, c_dev, C.c_void_p, c_dev, c_dev, c_dev], cint),
+    "bis_spmm": ([c_ctx, c_mat, cint, c_dev, c_dev], cint),
+    "bis_block_dot_to_slots": ([c_ctx, i64, cint, c_dev, c_dev, cint, c_dev], cint),
+    "bis_block_residual": ([c_ctx, cint, i64, cint] + [c_dev] * 6 + [cint] * 2, cint),
+    "bis_block_cg_update": ([c_ctx, cint, i64, cint] + [c_dev] * 5 + [cint] * 4 + [c_dev], cint),
+    "bis_block_cg_direction_x": ([c_ctx, i64, cint] + [c_dev] * 5 + [cint] * 3 + [c_dev], cint),
+    "bis_block_cg_status": ([c_ctx, cint, cint, cint, c_dev], cint),
 }
 
 _lib = None
@@ -374,6 +380,10 @@ class Context:
         l, u = c_mat(), c_mat()
         self.call("bis_matrix_split_triangular", A.h, C.byref(l), C.byref(u))
         return Matrix(self, l), Matrix(self, u)
+
+    def spmm(self, A: Matrix, X: int, Y: int, k: int):
+        """Y = A X for k right-hand sides (bis_spmm): X, Y device blocks of n x k doubles, row-major."""
+        self.call("bis_spmm", A.h, int(k), X, Y)
 
     # scalars -----------------------------------------------------------------
     def ilu0(self, A: Matrix, n: int, pivot_tolerance: float = 1e-8, pivot_replacement: float = 1e-4):

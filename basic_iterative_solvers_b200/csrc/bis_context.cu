@@ -179,6 +179,7 @@ extern "C" int bis_context_destroy(bis_context *c) {
     cudaFree(c->d_scalars);
     cudaFreeHost(c->h_scalars);
     cudaFree(c->d_partials);
+    cudaFree(c->d_block_partials);
     cudaFree(c->d_counter);
     cudaFree(c->d_errflag);
     cudaFree(c->d_barrier_word);

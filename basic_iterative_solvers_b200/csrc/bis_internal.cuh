@@ -156,6 +156,7 @@ struct bis_context {
     double *d_scalars = nullptr;         // BIS_NUM_SCALARS
     double *h_scalars = nullptr;         // pinned staging
     double *d_partials = nullptr;
+    double *d_block_partials = nullptr;  // [2*BIS_BLOCK_MAX_K][BIS_MAX_RED_BLOCKS]: multi-RHS reductions (bis_block.cu), on first use
     unsigned int *d_counter = nullptr;
     int *d_errflag = nullptr;            // set by kernels on watchdog expiry
     void *d_flush = nullptr;

@@ -46,6 +46,8 @@ def load() -> C.CDLL:
     lib.bis_host_gmres_update_g.restype = C.c_double
     lib.bis_host_solve.argtypes = ([C.c_void_p, C.c_char_p, C.c_int] + [C.c_void_p] * 3 + [C.c_int] * 3 +
                                    [C.c_void_p] * 2 + [C.c_int, C.c_double, C.c_int, C.c_int] + [C.c_void_p] * 5)
+    lib.bis_host_solve_block.argtypes = ([C.c_void_p, C.c_char_p, C.c_int] + [C.c_void_p] * 3 + [C.c_int] * 2 +
+                                         [C.c_void_p] * 2 + [C.c_int, C.c_double, C.c_int] + [C.c_void_p] * 7)
     lib.bis_host_bench_open.argtypes = [C.c_void_p, C.c_char_p, C.c_int, C.c_int, C.c_int]
     lib.bis_host_bench_open.restype = C.c_void_p
     lib.bis_host_bench_close.argtypes = [C.c_void_p]
@@ -195,6 +197,70 @@ def solve(ctx: capi.Context, method: str, precond: str = "none", *, crs=None, ma
     return SolveResult(hist[:cnt].copy(), float(od[1]), int(oi[0]), bool(oi[2]), int(oi[3]),
                        float(od[0]), xs, itime[1:cnt + 1].copy(), float(od[2]), float(od[3]),
                        float(od[4]), int(oi[4]))
+
+
+@dataclass
+class BlockSolveResult:
+    histories: list              # per column: residual norms ||r_0|| .. ||r_{iter_count}||
+    iter_counts: np.ndarray      # per column
+    converged: np.ndarray        # per column (bool)
+    final_true_residuals: np.ndarray   # per column ||b_j - A x*_j||
+    x_star: np.ndarray | None    # (n, k)
+    solve_time: float            # seconds: initial residual, iterations, read-backs
+    launches: int
+    iterations: int              # passes of the loop (the largest iter_count)
+
+
+def _solve_block(ctx, precond, crs, matrix_name, B, X0, max_iters, tol, want_x, timer_from):
+    lib = load()
+    B = np.ascontiguousarray(B, np.float64)
+    if B.ndim == 1:
+        B = B.reshape(-1, 1)
+    if B.ndim != 2:
+        raise ValueError("solve_block: B must be (n, k)")
+    n, k = B.shape
+    X0 = None if X0 is None else np.ascontiguousarray(np.reshape(X0, (n, k)), np.float64)
+    if crs is not None:
+        rp = np.ascontiguousarray(crs[0], np.int32)
+        col = np.ascontiguousarray(crs[1], np.int32)
+        val = np.ascontiguousarray(crs[2], np.float64)
+        if rp.size - 1 != n:
+            raise ValueError("solve_block: B has %d rows, the matrix %d" % (n, rp.size - 1))
+        name = None
+    else:
+        if matrix_name is None:
+            raise ValueError("solve_block: give crs= or matrix_name=")
+        rp = col = val = None
+        name = matrix_name.encode()
+    hist = np.zeros((k, 2 * MAX_ITERS))
+    its = np.zeros(k, np.int32)
+    conv = np.zeros(k, np.int32)
+    fres = np.zeros(k)
+    xs = np.zeros((n, k)) if want_x else None
+    od = np.zeros(4)
+    oi = np.zeros(4, np.int64)
+    rc = lib.bis_host_solve_block(ctx.h, name, n, _p(rp), _p(col), _p(val), k, PRECOND[precond], _p(B), _p(X0),
+                                  int(max_iters), float(tol), int(timer_from), _p(hist), _p(its), _p(conv), _p(fres),
+                                  _p(xs), _p(od), _p(oi))
+    if rc != 0:
+        raise capi.BisError(_err())
+    res = BlockSolveResult([hist[j, :its[j] + 1].copy() for j in range(k)], its.astype(np.int64), conv.astype(bool),
+                           fres, xs, float(od[0]), int(oi[0]), int(oi[2]))
+    return res, float(od[1]), int(oi[3])
+
+
+def solve_block(ctx: capi.Context, precond: str = "none", *, crs=None, matrix_name=None, B, X0=None,
+                max_iters: int = 0, tol: float = 0.0, want_x: bool = True) -> BlockSolveResult:
+    """CG on the k columns of B (an (n, k) array) with one matrix (host/methods/block_cg.hpp), precond "none"
+    or "j".  Every column runs the single-RHS CG's arithmetic and stop rule; the columns share one SpMM per
+    iteration.  X0: (n, k) or None (INIT_X_VAL).  max_iters <= 0 / tol <= 0 keep MAX_ITERS / TOL."""
+    return _solve_block(ctx, precond, crs, matrix_name, B, X0, max_iters, tol, want_x, 0)[0]
+
+
+def bench_block(ctx: capi.Context, matrix_name: str, B, precond: str = "none", warmup: int = 5, steps: int = 50):
+    """Measurement: exactly warmup + steps block-CG iterations (tolerance 0) on a named matrix; device time of
+    the last `steps` between CUDA events.  Returns (BlockSolveResult without x_star, timed ms, timed iterations)."""
+    return _solve_block(ctx, precond, None, matrix_name, B, None, warmup + steps, 0.0, False, warmup)
 
 
 def harness_trace(run_ahead: bool, max_iters: int, tol: float, decay: float):

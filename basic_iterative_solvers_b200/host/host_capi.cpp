@@ -2,6 +2,7 @@
 // the reference-shaped Solver/harness stack driven from plain C (ctypes in the
 // tests and bench.py).  Device work goes through the C-ABI of libbis_b200.so.
 #include "lu_factors.hpp"
+#include "methods/block_cg.hpp"
 #include "run.hpp"
 
 #include <cstring>
@@ -230,6 +231,87 @@ int bis_host_solve(bis_context *dev, const char *matrix_name, int n, const int *
     }
 }
 
+// CG on k right-hand sides with one matrix (methods/block_cg.hpp).  Matrix: host CRS arrays (rp != NULL) or a
+// generator / file name, as bis_host_solve.  B: n x k row-major host array; X0 likewise or NULL (INIT_X_VAL).
+// precond: none or jacobi.  max_iters <= 0 keeps MAX_ITERS; tol <= 0 keeps TOL.
+// Outputs per column j: history + j*2*MAX_ITERS (the residual norms, iter_count[j] + 1 of them),
+// iter_count[j], converged[j], final_res[j] = ||b_j - A x*_j||; x_star: n x k (may be NULL).
+// timer_from > 0: exactly max_iters iterations with tolerance 0, device time of iterations timer_from+1 ..
+// max_iters in out_dbl[1] (measurements).
+// out_dbl: [0] solve seconds (init residual, iterations, read-backs), [1] timed device ms.
+// out_int: [0] kernel launches of the solve, [1] rows n, [2] iterations of the loop, [3] timed iterations.
+int bis_host_solve_block(bis_context *dev, const char *matrix_name, int n, const int *rp, const int *col,
+                         const double *val, int k, int precond, const double *B, const double *X0, int max_iters,
+                         double tol, int timer_from, double *history, int *iter_count, int *converged,
+                         double *final_res, double *x_star, double *out_dbl, int64_t *out_int) {
+    try {
+        Args args;
+        args.matrix_file_name = matrix_name ? matrix_name : "in-memory";
+        args.method = SolverType::ConjugateGradient;
+        args.preconditioner = static_cast<PrecondType>(precond);
+        args.quiet = true;
+        if (!B) bis_fatal("block CG: B is required");
+        int perm_mode = 0;
+        BIS_OK(bis_context_get_option(dev, "perm_mode", &perm_mode));
+        if (perm_mode != 0) bis_fatal("block CG: perm_mode is not supported with several right-hand sides");
+        BlockCGSolver solver(&args, dev, k);
+        if (max_iters > 0) {
+            if (max_iters > MAX_ITERS) bis_fatal("max_iters exceeds MAX_ITERS");
+            solver.max_iters = max_iters;
+        }
+        if (tol > 0) solver.tolerance = tol;
+        if (timer_from > 0) {
+            if (timer_from >= solver.max_iters) bis_fatal("block CG: timer_from must be below max_iters");
+            solver.tolerance = 0.0;   // never stop early: exactly max_iters iterations
+        }
+        std::unique_ptr<MatrixCRS> A;
+        std::unique_ptr<DeviceCRS> dA;
+        if (rp) {
+            A = std::make_unique<MatrixCRS>(n, n, rp[n]);
+            std::memcpy(A->row_ptr, rp, sizeof(int) * (n + 1));
+            std::memcpy(A->col, col, sizeof(int) * rp[n]);
+            std::memcpy(A->val, val, sizeof(double) * rp[n]);
+            dA = upload_crs(dev, A.get());
+            A.reset();
+        } else {
+            obtain_matrix(&args, dev, A, dA);
+            if (A) {
+                dA = upload_crs(dev, A.get());
+                A.reset();
+            }
+        }
+        if (n > 0 && dA->n_rows != n) bis_fatal("block CG: B has " + std::to_string(n) + " rows, the matrix " +
+                                               std::to_string(dA->n_rows));
+        int64_t info0[8], info1[8];
+        BIS_OK(bis_context_info(dev, info0));
+        Stopwatch w;
+        w.start();
+        solver.setup(std::move(dA), B, X0);
+        double timed_ms = 0.0;
+        int timed_iters = 0;
+        solver.run(timer_from, &timed_ms, &timed_iters);
+        out_dbl[0] = w.check();
+        out_dbl[1] = timed_ms;
+        BIS_OK(bis_context_info(dev, info1));
+        const std::vector<double> fr = solver.true_residuals();
+        for (int j = 0; j < k; ++j) {
+            const std::vector<double> &h = solver.col_history[(size_t)j];
+            for (size_t i = 0; i < h.size() && i < (size_t)(2 * MAX_ITERS); ++i) history[(size_t)j * 2 * MAX_ITERS + i] = h[i];
+            iter_count[j] = solver.col_iters[(size_t)j];
+            converged[j] = solver.col_converged[(size_t)j];
+            final_res[j] = fr[(size_t)j];
+        }
+        if (x_star) BIS_OK(bis_vector_download(dev, x_star, solver.X_old, solver.N * k));
+        out_int[0] = info1[3] - info0[3];
+        out_int[1] = solver.N;
+        out_int[2] = solver.iter_count;
+        out_int[3] = timed_iters;
+        return 0;
+    } catch (const std::exception &e) {
+        g_host_err = e.what();
+        return 1;
+    }
+}
 
 // ---- measurement sessions (bench.py) ----------------------------------------------
 // A session owns one Solver on one named matrix.  Two timed regions:

@@ -427,6 +427,71 @@ int bis_gmres_update_x(bis_context *ctx, int64_t n, int k, const double *V,
                        const double *y /* [host] */, double *x,
                        const double *x_old, double *Vy);
 
+/* ---- multiple right-hand sides -----------------------------------------
+ * New in the build: the reference solves one right-hand side at a time.
+ * Several systems with the same matrix (load cases, sources, sweeps over b)
+ * share ONE pass over the matrix per iteration.  Single-GPU contexts only.
+ *
+ * Layout: a block of k vectors (1 <= k <= BIS_BLOCK_MAX_K) is an n x k
+ * ROW-MAJOR device array, element (i, j) at V[i*k + j], allocated with
+ * bis_vector_alloc(ctx, n*k) (16-byte aligned; every block argument must be).
+ * A numpy / torch (n, k) C-contiguous array uploads as is.  Column j's
+ * scalars live in slots slot0 + j; slot0 + k > BIS_NUM_SCALARS is an error.
+ *
+ * Every column is bit-identical to the single-vector entry point it batches:
+ * bis_spmm to native_spmv (products rounded separately, added in storage
+ * order; = bis_spmv wherever that takes the TMA-tile or windowed variant),
+ * the streaming kernels to bis_dot_to_slot / bis_subtract_vectors /
+ * bis_elemwise_div_vectors / bis_cg_update / bis_cg_direction_x (same rows
+ * per block, same accumulation order, same reduction tree).  All are
+ * enqueue-only (graph-recordable).  They fail on a distributed context, k
+ * outside [1, 16], a block argument that is not 16-byte aligned and a matrix
+ * without CRS arrays (option factor_keep_crs = 0).
+ *
+ * `state` [dev] of a block CG: 3k doubles, [0,k) stop thresholds
+ * tol*||r0_j||, [k,2k) active flags (1.0 / 0.0), [2k,3k) iterations done;
+ * NULL = every column active.  A column that is not active is frozen: its
+ * vectors and slots are not written, except that the direction step carries
+ * its x through (X_new = X_old), so the final iterate of every column is
+ * always in the X_new of the last step. */
+#define BIS_BLOCK_MAX_K 16
+/* Y = A X, X: n_cols x k, Y: n_rows x k.  Counted in the "spmv" profile
+ * family, NVTX range "spmm". */
+int bis_spmm(bis_context *ctx, const bis_matrix *A, int k, const double *X /* [dev] */,
+             double *Y /* [dev] */);
+/* slot0 + j <- (A_j, B_j) for every column j (active ones only if state). */
+int bis_block_dot_to_slots(bis_context *ctx, int64_t n, int k, const double *A,
+                           const double *B, int slot0, const double *state);
+/* Initial residual of a block CG (cg.hpp:100-120 per column): R = B - AX,
+ * Z = M^-1 R (precond NONE: copy, JACOBI: R / A_D), P = Z if P != NULL,
+ * slot_rz0 + j <- (r_j, z_j), slot_rr0 + j <- (r_j, r_j). */
+int bis_block_residual(bis_context *ctx, int precond, int64_t n, int k,
+                       const double *AX, const double *B, const double *A_D,
+                       double *R, double *Z, double *P, int slot_rz0,
+                       int slot_rr0);
+/* bis_cg_update (x_new = NULL) per column: alpha_j = s[rz0+j]/s[pAp0+j];
+ * R_new = R_old - alpha AP; Z_new = R_new or R_new / A_D; s[rr0+j] <-
+ * (r,r); s[rz_new0+j] <- (r,z).  Precond NONE or JACOBI only. */
+int bis_block_cg_update(bis_context *ctx, int precond, int64_t n, int k,
+                        double *R_new, const double *R_old, const double *AP,
+                        double *Z_new, const double *A_D, int slot_rz0,
+                        int slot_pAp0, int slot_rr0, int slot_rz_new0,
+                        const double *state);
+/* bis_cg_direction_x per column: X_new = X_old + alpha P_old, P_new = Z_new
+ * + beta P_old (inactive columns: X_new = X_old, P_new untouched). */
+int bis_block_cg_direction_x(bis_context *ctx, int64_t n, int k, double *P_new,
+                             const double *Z_new, const double *P_old,
+                             double *X_new, const double *X_old,
+                             int slot_rz_new0, int slot_rz0, int slot_pAp0,
+                             const double *state);
+/* Start of a block-CG iteration: the stop rule of the harness
+ * (solver.hpp:173-191) on the device, latched for the whole iteration.  An
+ * active column that has run >= 1 iteration stops when sqrt(s[rr0+j]) <
+ * threshold, > DBL_MAX or NaN; one that has run max_iters stops; every
+ * column still active counts the iteration. */
+int bis_block_cg_status(bis_context *ctx, int k, int slot_rr0, int max_iters,
+                        double *state /* [dev] */);
+
 #ifdef __cplusplus
 }
 #endif
