@@ -421,6 +421,8 @@ extern "C" int bis_context_get_option(bis_context *c, const char *key, int *valu
     else if (k == "perm_mode") *value = c->opt_perm_mode;
     else if (k == "spmv_vdict") *value = c->opt_spmv_vdict;
     else if (k == "spmv_value_bytes") *value = c->last_spmv_value_bytes;   // read-only: what the last windowed SpMV streamed per nonzero
+    else if (k == "spmv_stream_mb")      // read-only: the last windowed SpMV's compulsory bytes, in 1e6 bytes (an int holds no byte count)
+        *value = (int)((c->last_spmv_stream_bytes + 500000) / 1000000);
     else if (k == "factor_keep_crs") *value = c->opt_factor_keep_crs;
     else if (k == "spmv_variant") *value = c->opt_spmv_variant;
     else if (k == "trsv_variant") *value = c->opt_trsv_variant;

@@ -205,9 +205,10 @@ struct bis_context {
     int opt_trsv_debug = 0;     // dump per-row timestamps of each solve to $BIS_TRSV_DEBUG_FILE
     int opt_spmv_rows = 0;      // TMA variant: rows per tile (0 auto)
     int opt_spmv_stages = 0;    // TMA variant: max stages (0 auto)
-    int opt_spmv_vdict = 0;     // windowed SpMV: 1 = stream 1-byte value indices when the matrix has <= 256 distinct values (lossless; off by
-                                // default: 12 % faster at HPCG-512, + 1 byte per nonzero of memory, see DESIGN.md 3.1)
+    int opt_spmv_vdict = 1;     // windowed SpMV: 1 = stream 1-byte value indices when the matrix has <= 256 distinct values (lossless,
+                                // + 1 byte per nonzero of memory; 0 = stream the values; see DESIGN.md 3.1)
     int last_spmv_value_bytes = 8;   // bytes per nonzero the last windowed SpMV streamed for the values (8 or 1)
+    int64_t last_spmv_stream_bytes = 0;   // compulsory HBM bytes of the last windowed SpMV launch (its format's byte model)
     int opt_wave_cluster = 8;   // stencil wavefront: planes per thread-block cluster (1: no clusters, every hand-over through L2)
     int opt_wave_backoff_ns = 0;      // ... nanoseconds a plane fed through L2 falls back after it had to poll (clusters only)
     int wave_cluster_used = 0;  // ... what the last solve ran with

@@ -23,6 +23,8 @@
 #include "bis_spmv_tma.cuh"
 #include "bis_spmv_win.cuh"
 #include <algorithm>
+#include <cstdio>
+#include <cstdlib>
 #include <cstring>
 #include <vector>
 
@@ -51,10 +53,12 @@ struct SpmvIn {
 };
 
 // Epilogues.  load(r) fetches the per-row operands (issued BEFORE the row's sum is available so
-// that their latency overlaps the tile wait / row walk); operator() consumes them.
+// that their latency overlaps the tile wait / row walk); operator() consumes them.  vectors(x): how
+// many n-vectors the epilogue reads or writes besides x (the byte model of spmv_stream_mb).
 struct EpiStore {
     static constexpr int NRED = 0;
     double *y;
+    int vectors(const double *) const { return 1; }
     __device__ __forceinline__ EpiPre load(int64_t) const { return EpiPre{0.0, 0.0, 0.0}; }
     __device__ __forceinline__ void operator()(int64_t r, double s, const EpiPre &, double *) const { y[r] = s; }
 };
@@ -62,6 +66,7 @@ struct EpiDot {
     static constexpr int NRED = 2;
     double *y;
     const double *w;
+    int vectors(const double *x) const { return 1 + (w != x ? 1 : 0); }
     __device__ __forceinline__ EpiPre load(int64_t r) const { return EpiPre{w[r], 0.0, 0.0}; }
     __device__ __forceinline__ void operator()(int64_t r, double s, const EpiPre &p, double *acc) const {
         y[r] = s;
@@ -74,6 +79,7 @@ struct EpiResid {
     const double *b;
     double *res;
     double *tmp;
+    int vectors(const double *) const { return 2 + (tmp ? 1 : 0); }
     __device__ __forceinline__ EpiPre load(int64_t r) const { return EpiPre{b[r], 0.0, 0.0}; }
     __device__ __forceinline__ void operator()(int64_t r, double s, const EpiPre &p, double *acc) const {
         if (tmp) tmp[r] = s;
@@ -86,6 +92,7 @@ struct EpiJacobi {
     static constexpr int NRED = 0;
     const double *D, *b, *x_old;
     double *x_new;
+    int vectors(const double *) const { return 3; }
     __device__ __forceinline__ EpiPre load(int64_t r) const { return EpiPre{D[r], x_old[r], b[r]}; }
     __device__ __forceinline__ void operator()(int64_t r, double s, const EpiPre &p, double *) const {
         double scaled = mul_rn(p.a, p.b);
@@ -101,6 +108,7 @@ struct EpiJacobiResid {
     const double *D, *b, *x_old;
     double *x_new;
     double *res;       // may be null
+    int vectors(const double *) const { return 3 + (res ? 1 : 0); }
     __device__ __forceinline__ EpiPre load(int64_t r) const { return EpiPre{D[r], x_old[r], b[r]}; }
     __device__ __forceinline__ void operator()(int64_t r, double s, const EpiPre &p, double *acc) const {
         const double scaled = mul_rn(p.a, p.b);
@@ -115,6 +123,7 @@ struct EpiSub {
     static constexpr int NRED = 0;
     const double *b;
     double *out;
+    int vectors(const double *) const { return 2; }
     __device__ __forceinline__ EpiPre load(int64_t r) const { return EpiPre{b[r], 0.0, 0.0}; }
     __device__ __forceinline__ void operator()(int64_t r, double s, const EpiPre &p, double *) const {
         out[r] = sub_rn(p.a, s);
@@ -128,6 +137,7 @@ struct EpiTwoStage {
     const double *D_inv;
     double *w_out;
     double *out;
+    int vectors(const double *) const { return 4; }     // out is read and written
     __device__ __forceinline__ EpiPre load(int64_t r) const { return EpiPre{D_inv[r], out[r], 0.0}; }
     __device__ __forceinline__ void operator()(int64_t r, double s, const EpiPre &p, double *) const {
         const double t = mul_rn(mul_rn(p.a, -1.0), s);
@@ -447,6 +457,14 @@ int win_build_dict(bis_context *c, const bis_matrix *A) {
     std::sort(pats.begin(), pats.end());
     double dict[256] = {};
     for (size_t i = 0; i < pats.size(); ++i) memcpy(&dict[i], &pats[i], sizeof(double));
+    // the index array is an acceleration structure: it is built only while an eighth of the device memory stays free
+    // after it, so that what the solver allocates later (vectors, triangular factors) is not crowded out by it
+    size_t fr = 0, tot = 0;
+    if (cudaMemGetInfo(&fr, &tot) != cudaSuccess || (size_t)A->nnz + 32 + tot / 8 > fr) {
+        cudaGetLastError();
+        cudaFree(d_state);
+        return 0;
+    }
     if (cudaMalloc(&w.d_vidx, (size_t)A->nnz + 32) != cudaSuccess) {     // no room for the index array: the values are streamed
         cudaGetLastError();
         w.d_vidx = nullptr;
@@ -724,8 +742,18 @@ int launch_win(bis_context *c, const bis_matrix *A, const WinPlan &p, const doub
     in.val_region = dict ? w.cap : w.cap * 8;
     in.amask = dict ? 15 : 7;
     c->last_spmv_value_bytes = dict ? 1 : 8;
+    // the launch's compulsory HBM bytes in this format: value (8 B or a 1-byte dictionary index) and 16-bit column id
+    // per nonzero, the row_ptr slices, x once, and the vectors of the epilogue (the x windows are re-read from L2)
+    c->last_spmv_stream_bytes = (int64_t)(dict ? 3 : 10) * A->nnz + (int64_t)A->rp_bytes * (A->n_rows + 1) +
+                                8 * (A->n_cols + (int64_t)epi.vectors(x) * A->n_rows);
 #ifdef BIS_PERF_DEBUG
     in.debug = c->opt_spmv_debug;
+    in.stamps = nullptr;
+    const char *stamp_file = (c->opt_spmv_debug & 4) ? getenv("BIS_SPMV_STAMPS") : nullptr;
+    if (stamp_file) {
+        BIS_CUDA(bis_cuda_malloc(&in.stamps, sizeof(unsigned long long) * WIN_NSTAMP));
+        BIS_CUDA(cudaMemsetAsync(in.stamps, 0, sizeof(unsigned long long) * WIN_NSTAMP, c->stream));
+    }
 #endif
     ra.finalize = 1;
     ra.block_offset = 0;
@@ -754,6 +782,19 @@ int launch_win(bis_context *c, const bis_matrix *A, const WinPlan &p, const doub
         kern<<<(unsigned)grid, threads, p.smem_bytes, c->stream>>>(in, epi, ra, NoHaloFuse{});
     }
     BIS_LAUNCH_CHECK(c);
+#ifdef BIS_PERF_DEBUG
+    if (in.stamps) {
+        unsigned long long h[WIN_NSTAMP];
+        BIS_CUDA(cudaMemcpyAsync(h, in.stamps, sizeof h, cudaMemcpyDeviceToHost, c->stream));
+        BIS_CUDA(cudaStreamSynchronize(c->stream));
+        h[WIN_NSTAMP - 1] = (unsigned long long)grid;
+        if (FILE *f = fopen(stamp_file, "ab")) {
+            fwrite(h, sizeof(unsigned long long), WIN_NSTAMP, f);
+            fclose(f);
+        }
+        cudaFree(in.stamps);
+    }
+#endif
     return 0;
 }
 

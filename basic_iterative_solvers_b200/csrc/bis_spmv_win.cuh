@@ -317,7 +317,9 @@ struct SpmvWinIn {
     int ngroups;                  // consumer groups (tile s is computed by group s % ngroups); nstage is a multiple of it
     int stage_bytes;
 #ifdef BIS_PERF_DEBUG
-    int debug;                    // perf experiments only (results invalid): 1 = consumers skip the row walk, 2 = no x-window copies
+    int debug;                    // perf experiments only: 1 = consumers skip the row walk, 2 = no x-window copies (results
+                                  // invalid); 4 = per-role cycle counters into `stamps` (results valid, see WinStamp)
+    unsigned long long *stamps;   // [WIN_NSTAMP], summed over the CTAs
 #endif
 };
 #ifdef BIS_PERF_DEBUG
@@ -325,6 +327,23 @@ struct SpmvWinIn {
 #else
 #define BIS_WIN_DEBUG(in, bit) 0
 #endif
+
+// Per-role cycle counters of the -DBIS_PERF_DEBUG build (spmv_debug bit 4; tools/run_spmv_stamps.py).  Producer: lane 0
+// of the producer warp; consumers: lane 0 of every consumer warp (a warp's lanes run the same steps).  SM cycles
+// (clock64): the phases of a tile are a few hundred cycles, below what the global timer resolves.
+enum WinStamp {
+    WS_P_EMPTY = 0,     // producer: waiting on a stage's `empty` barrier
+    WS_P_ISSUE,         // producer: proxy fence, expect_tx and the bulk-copy instructions of a tile
+    WS_P_TILES,         // producer: tiles issued
+    WS_P_TOTAL,         // producer: whole tile loop
+    WS_C_ORDER,         // consumers: waiting on the next tile id (order table load)
+    WS_C_FULL,          // consumers: waiting on a stage's `full` barrier
+    WS_C_EPILOAD,       // consumers: waiting on the epilogue operand load issued before the `full` wait
+    WS_C_WALK,          // consumers: row walk and epilogue stores
+    WS_C_TILES,         // consumers: tiles, summed over warps
+    WS_C_TOTAL,         // consumers: whole tile loop, summed over warps
+    WIN_NSTAMP = 16     // the host writes the launch's grid size into the last slot
+};
 
 // stage layout: [val cap*8 | vidx cap][xwin xcap*8][rp (R+4)*8][lidx cap*2], every part 16-byte aligned
 constexpr int WIN_MAX_THREADS = 544;   // consumer groups (R x nstage <= 512) + the producer warp
@@ -482,6 +501,10 @@ spmv_win_kernel(SpmvWinIn in, Epi epi, RedArgs ra, typename std::conditional<DIS
             }
         };
         [[maybe_unused]] bool halo_seen = false;
+#ifdef BIS_PERF_DEBUG
+        long long pst[4] = {0, 0, 0, 0};
+        const long long t_p0 = clock64();
+#endif
         auto issue = [&](int s, const Desc &d) {
             if constexpr (DIST) {
                 // first tile of this CTA that reads ghosts: the senders' values must have landed
@@ -541,15 +564,25 @@ spmv_win_kernel(SpmvWinIn in, Epi epi, RedArgs ra, typename std::conditional<DIS
             uint32_t total = bytes;
 #pragma unroll
             for (int o = 16; o > 0; o >>= 1) total += __shfl_xor_sync(0xffffffffu, total, o);
+#ifdef BIS_PERF_DEBUG
+            const long long t_w0 = clock64();
+#endif
             // the stage must have been released by every consumer warp
-            if (s >= in.nstage) {
-                tma::mbar_wait(&empty[st], (uint32_t)(((s / in.nstage) - 1) & 1));
-                tma::fence_reads_before_bulk_write();
-            }
+            if (s >= in.nstage) tma::mbar_wait(&empty[st], (uint32_t)(((s / in.nstage) - 1) & 1));
+#ifdef BIS_PERF_DEBUG
+            const long long t_w1 = clock64();
+#endif
+            if (s >= in.nstage) tma::fence_reads_before_bulk_write();
             unsigned char *sb = stages + (size_t)st * in.stage_bytes;
             if (lane == 0) tma::mbar_expect_tx(&full[st], total);
             __syncwarp();
             if (bytes) tma::bulk_g2s(sb + dst, src, bytes, &full[st], lane < 3 ? pol_stream : pol_keep);
+#ifdef BIS_PERF_DEBUG
+            __syncwarp();
+            pst[WS_P_EMPTY] += t_w1 - t_w0;
+            pst[WS_P_ISSUE] += clock64() - t_w1;
+            pst[WS_P_TILES] += 1;
+#endif
         };
         constexpr int PDEPTH = 4;
         int tq[2 * PDEPTH];     // order entries of tiles s .. s + 7
@@ -569,6 +602,12 @@ spmv_win_kernel(SpmvWinIn in, Epi epi, RedArgs ra, typename std::conditional<DIS
                 tq[u] = load_order(s + 2 * PDEPTH);
             }
         }
+#ifdef BIS_PERF_DEBUG
+        if (in.stamps && lane == 0) {
+            pst[WS_P_TOTAL] = clock64() - t_p0;
+            for (int q = 0; q < 4; ++q) atomicAdd(in.stamps + q, (unsigned long long)pst[q]);
+        }
+#endif
     } else {
         [[maybe_unused]] int cur_slab = 0;
         // the slab-end partial of a fused reduction is formed by the consumer warps alone (the producer
@@ -603,8 +642,23 @@ spmv_win_kernel(SpmvWinIn in, Epi epi, RedArgs ra, typename std::conditional<DIS
             }
         };
         int raw_next = group < my_tiles ? in.ord.order[seq.pos(in.ord, (int)blockIdx.x, group)] : 0;
+#ifdef BIS_PERF_DEBUG
+        long long cst[6] = {0, 0, 0, 0, 0, 0};     // WS_C_ORDER .. WS_C_TOTAL
+        const long long t_c0 = clock64();
+#endif
         for (int s = group; s < my_tiles; s += in.ngroups) {
             const int st = s % in.nstage;
+#ifdef BIS_PERF_DEBUG
+            long long t_a = clock64();
+            if (in.stamps) {     // consume the tile id now, so that its wait is counted here
+                int v;
+                asm volatile("add.s32 %0, %1, 1;" : "=r"(v) : "r"(raw_next));
+                asm volatile("" ::"r"(v));
+                const long long t_b = clock64();
+                cst[0] += t_b - t_a;
+                t_a = t_b;
+            }
+#endif
             const int tile = raw_next & ~WIN_ORDER_GHOST;
             if constexpr (Epi::NRED > 0) {
                 const int slab = seq.slab_of(s);
@@ -622,7 +676,24 @@ spmv_win_kernel(SpmvWinIn in, Epi epi, RedArgs ra, typename std::conditional<DIS
                 reinterpret_cast<const unsigned short *>(reinterpret_cast<const unsigned char *>(srp) + (size_t)(R + 4) * 8);
             EpiPre pre{0.0, 0.0, 0.0};
             if (row < in.n_rows) pre = epi.load(row);   // in flight during the wait and the row walk
+#ifdef BIS_PERF_DEBUG
+            const long long t_f0 = clock64();
+#endif
             tma::mbar_wait(&full[st], (uint32_t)((s / in.nstage) & 1));
+#ifdef BIS_PERF_DEBUG
+            long long t_f1 = clock64();
+            if (in.stamps) {
+                cst[1] += t_f1 - t_f0;
+                double v;
+                asm volatile("add.f64 %0, %1, %2;" : "=d"(v) : "d"(pre.a), "d"(pre.b));
+                asm volatile("add.f64 %0, %0, %1;" : "+d"(v) : "d"(pre.c));
+                asm volatile("" ::"d"(v));
+                const long long t_f2 = clock64();
+                cst[2] += t_f2 - t_f1;
+                t_f1 = t_f2;
+            }
+            (void)t_a;
+#endif
             if (row < in.n_rows && !BIS_WIN_DEBUG(in, 1)) {
                 const int64_t base = (int64_t)srp[0] & ~(int64_t)in.amask;
                 const int ks = (int)((int64_t)srp[tid_g] - base);
@@ -656,8 +727,18 @@ spmv_win_kernel(SpmvWinIn in, Epi epi, RedArgs ra, typename std::conditional<DIS
                 epi(row, sum, pre, acc);
             }
             __syncwarp();
+#ifdef BIS_PERF_DEBUG
+            cst[3] += clock64() - t_f1;
+            cst[4] += 1;
+#endif
             if (lane == 0) tma::mbar_arrive(&empty[st]);
         }
+#ifdef BIS_PERF_DEBUG
+        if (in.stamps && lane == 0) {
+            cst[5] = clock64() - t_c0;
+            for (int q = 0; q < 6; ++q) atomicAdd(in.stamps + WS_C_ORDER + q, (unsigned long long)cst[q]);
+        }
+#endif
         if constexpr (Epi::NRED > 0) {
             while (cur_slab < in.ord.n_slab) close_slab(cur_slab++);
         }

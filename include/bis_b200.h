@@ -100,10 +100,12 @@ int bis_flush_l2(bis_context *ctx);
 /* Tuning knobs (all have defaults): key = "spmv_variant" (0 auto, 1 vector
  * CRS, 2 TMA-staged tiles + gathers, 3 windowed x), "spmv_lanes" (0 auto,
  * 2..32), "trsv_variant" (0 auto, 1 launch per level, 2 level counters,
- * 3 dataflow, 4 chains, 5 stencil wavefront), "spmv_vdict" (default 0; 1: the
+ * 3 dataflow, 4 chains, 5 stencil wavefront), "spmv_vdict" (default 1: the
  * windowed SpMV of a matrix with at most 256 distinct values streams a 1-byte
- * index per nonzero instead of the 8-byte value -- lossless, same bits;
- * "spmv_value_bytes" reads back what the last launch streamed), "wave_cluster" (stencil
+ * index per nonzero instead of the 8-byte value -- lossless, same bits, + 1 byte
+ * per nonzero of memory; 0: the values are streamed;
+ * "spmv_value_bytes" reads back what the last launch streamed, "spmv_stream_mb" its
+ * compulsory HBM bytes in units of 1e6 from the format's byte model), "wave_cluster" (stencil
  * wavefront: planes per thread-block cluster, 1 / 2 / 4 / 8 (default) / 16;
  * 1 = every plane-to-plane hand-over through L2), "perm_mode" (0 none,
  * 1 multicolouring, 2 BFS levels, 3 reverse Cuthill-McKee, 4 Cuthill-McKee:

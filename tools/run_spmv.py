@@ -31,4 +31,7 @@ with capi.Context(0) as ctx:
     for _ in range(reps):
         launch()
     ms = ctx.timer_stop() / reps
-    print(f"HPCG-{n} {sys.argv[3:]}: {ms:.3f} ms  {A.spmv_bytes()/ms/1e6:.1f} GB/s")
+    # the windowed kernel's own compulsory bytes, from its format's byte model (C library, option spmv_stream_mb)
+    own = ctx.get_option("spmv_stream_mb") * 1e6
+    print(f"HPCG-{n} {sys.argv[3:]}: {ms:.3f} ms  {A.spmv_bytes()/ms/1e6:.1f} GB/s CRS-equivalent  "
+          f"own {own/1e9:.2f} GB/launch ({ctx.get_option('spmv_value_bytes')} B values) {own/ms/1e6:.1f} GB/s")
