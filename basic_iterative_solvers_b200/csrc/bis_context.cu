@@ -425,6 +425,8 @@ extern "C" int bis_context_get_option(bis_context *c, const char *key, int *valu
         *value = (int)((c->last_spmv_stream_bytes + 500000) / 1000000);
     else if (k == "factor_keep_crs") *value = c->opt_factor_keep_crs;
     else if (k == "spmv_variant") *value = c->opt_spmv_variant;
+    else if (k == "spmv_lanes") *value = c->opt_spmv_lanes;
+    else if (k == "vector_cache") *value = c->opt_vector_cache;
     else if (k == "trsv_variant") *value = c->opt_trsv_variant;
     else if (k == "spmv_fused") *value = c->opt_spmv_fused;
     else if (k == "dist_p2p") *value = c->opt_dist_p2p;

@@ -513,7 +513,8 @@ extern "C" int bis_matrix_generate_anderson(bis_context *c, int lx, int ly, int 
     BIS_REQUIRE(c && out, "null argument");
     BIS_REQUIRE(lx >= 1 && ly >= 1 && lz >= 1, "bis_matrix_generate_anderson: bad lattice");
     const int64_t n = (int64_t)lx * ly * lz;
-    BIS_REQUIRE(n < INT32_MAX / 8, "bis_matrix_generate_anderson: lattice too large for 32-bit ids");
+    // row_ptr is 64-bit and the fill kernels index in 64 bits: only the column ids limit the lattice
+    BIS_REQUIRE(n < INT32_MAX, "bis_matrix_generate_anderson: %lld sites exceed 32-bit column ids", (long long)n);
     BIS_CUDA(cudaSetDevice(c->device));
     bis_vector_cache_trim(c);
     int64_t rb = 0, re = n;

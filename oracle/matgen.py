@@ -73,6 +73,11 @@ def hpcg_nnz(nx, ny=None, nz=None):
     return (3 * nx - 2) * (3 * ny - 2) * (3 * nz - 2)
 
 
+def anderson_diagonal(rows: np.ndarray, ranpot: float = 5.0, seed: int = 1) -> np.ndarray:
+    """on-site potential of the given rows: ranpot * U(-1, 1)"""
+    return ranpot * (2.0 * splitmix64_unit(seed, rows) - 1.0)
+
+
 def anderson(lx: int, ly: int, lz: int, ranpot: float = 5.0, t: float = 1.0,
              seed: int = 1, periodic: bool = False, row_begin: int = 0,
              row_end: int | None = None):
@@ -86,7 +91,7 @@ def anderson(lx: int, ly: int, lz: int, ranpot: float = 5.0, t: float = 1.0,
     cols = np.empty((m, 7), dtype=np.int64)
     valid = np.empty((m, 7), dtype=bool)
     vals = np.empty((m, 7), dtype=np.float64)
-    diag = ranpot * (2.0 * splitmix64_unit(seed, rows) - 1.0)
+    diag = anderson_diagonal(rows, ranpot, seed)
     steps = [(0, 0, -1), (0, -1, 0), (-1, 0, 0), (0, 0, 0), (1, 0, 0), (0, 1, 0), (0, 0, 1)]
     for k, (dx, dy, dz) in enumerate(steps):
         xx, yy, zz = x + dx, y + dy, z + dz

@@ -104,6 +104,151 @@ def sptrsv_inplace(rp, col, val, D, xb, backward=False):
     return x
 
 
+# ---- slab-wise application ----------------------------------------------------------------------------
+# A matrix whose nonzeros do not fit the oracle's int row_ptr is applied one row slab [rb, re) at a time.  A
+# slab comes as CRS with a row_ptr that starts at 0 (int32 for any slab of moderate height) and its columns
+# rebased to rb.  The unchanged C loops then run on views of the full vectors that start at row rb (x[rb:],
+# y[rb:], D[rb:], b[rb:]): a negative rebased column reads an earlier row through the view, and every row gets
+# the products, sums and roundings of the whole-matrix call.  Rebased to its own first row, every interior
+# slab of an HPCG grid has the same local structure, so three generated templates (first, interior, last)
+# serve the whole matrix.
+
+def rebase(rp, col, val, row_begin):
+    """a slab's CRS from matgen (global columns) with its columns made relative to row_begin"""
+    rp = np.ascontiguousarray(rp, dtype=np.int32)
+    col = np.ascontiguousarray(np.asarray(col, np.int64) - int(row_begin), dtype=np.int32)
+    return _crs(rp, col, val)
+
+
+def split_rebased(rp, col, val):
+    """(L, U, diag) of a rebased slab: strictly lower / upper parts as (rp, col, val), entries in storage order
+    exactly as o_split_strict keeps them; diag[i] is the last diagonal entry of row i (o_split_strict's A_D)"""
+    rp = np.asarray(rp, np.int64)
+    m = rp.size - 1
+    cnt = np.diff(rp)
+    rows = np.repeat(np.arange(m, dtype=np.int64), cnt)
+    col = np.asarray(col[:rp[-1]], np.int64)
+    val = np.asarray(val[:rp[-1]])
+    out = []
+    for keep in (col < rows, col > rows):
+        t_rp = np.zeros(m + 1, np.int32)
+        np.cumsum(np.bincount(rows[keep], minlength=m), out=t_rp[1:])
+        out.append(_crs(t_rp, col[keep].astype(np.int32), val[keep]))
+    diag = np.zeros(m)
+    on = col == rows
+    diag[rows[on]] = val[on]
+    return out[0], out[1], diag
+
+
+class GeneratedSlabs:
+    """Row slabs of `slab_rows` rows, each generated by gen(row_begin, row_end) -> (rp, col, val)"""
+
+    def __init__(self, gen, n, slab_rows):
+        self.gen, self.n = gen, n
+        self.bounds = [(rb, min(rb + slab_rows, n)) for rb in range(0, n, slab_rows)]
+
+    def crs(self, rb, re):
+        return rebase(*self.gen(rb, re), rb)
+
+    def split(self, rb, re):
+        return split_rebased(*self.crs(rb, re))
+
+
+class TemplatedSlabs:
+    """Row slabs of `planes` grid planes of a stencil matrix whose rebased structure and off-diagonal values
+    are the same in every interior slab, served from at most three templates generated by gen(row_begin,
+    row_end): the first slab, the interior ones and the last.  diagonal(rows), when given, supplies the
+    row-dependent diagonal values that are written into a copy of the template."""
+
+    def __init__(self, gen, n, plane, planes, diagonal=None):
+        self.n = n
+        self.diagonal = diagonal
+        self.bounds = [(rb, min(rb + planes * plane, n)) for rb in range(0, n, planes * plane)]
+        self._crs, self._split, self._dpos = {}, {}, {}
+        for rb, re in self.bounds:
+            key = self._key(rb, re)
+            if key not in self._crs:
+                self._crs[key] = rebase(*gen(rb, re), rb)
+                if diagonal is not None:
+                    rp, col, _ = self._crs[key]
+                    rows = np.repeat(np.arange(re - rb), np.diff(rp))
+                    pos = np.flatnonzero(col[:rp[-1]] == rows)
+                    assert np.array_equal(rows[pos], np.arange(re - rb)), "one diagonal entry per row"
+                    self._dpos[key] = pos
+
+    def _key(self, rb, re):
+        return rb == 0, re == self.n, re - rb
+
+    def crs(self, rb, re):
+        key = self._key(rb, re)
+        if self.diagonal is None:
+            return self._crs[key]
+        rp, col, val = self._crs[key]
+        val = val.copy()
+        val[self._dpos[key]] = self.diagonal(np.arange(rb, re, dtype=np.int64))
+        return rp, col, val
+
+    def split(self, rb, re):
+        if self.diagonal is not None:
+            return split_rebased(*self.crs(rb, re))
+        key = self._key(rb, re)
+        if key not in self._split:
+            self._split[key] = split_rebased(*self._crs[key])
+        return self._split[key]
+
+
+def hpcg_slabs(nx, ny, nz, planes):
+    from . import matgen
+    return TemplatedSlabs(lambda rb, re: matgen.hpcg(nx, ny, nz, rb, re), nx * ny * nz, nx * ny, planes)
+
+
+def anderson_slabs(lx, ly, lz, planes, ranpot=5.0, t=1.0, seed=1, periodic=False):
+    from . import matgen
+    return TemplatedSlabs(lambda rb, re: matgen.anderson(lx, ly, lz, ranpot, t, seed, periodic, rb, re),
+                          lx * ly * lz, lx * ly, planes, lambda rows: matgen.anderson_diagonal(rows, ranpot, seed))
+
+
+def spmv_slab_into(rp, col, val, x, y, row_begin):
+    """y[row_begin : row_begin + m] = rows of a rebased slab applied to the full x"""
+    m = rp.size - 1
+    load().o_spmv(m, rp, col, val, x[row_begin:], y[row_begin:row_begin + m])
+
+
+def spmv_slabwise(slabs, x, threads=None):
+    """y = A x slab by slab (slabs: GeneratedSlabs or HpcgSlabs); slabs are independent and the C loop runs
+    outside the GIL, so they are spread over threads"""
+    from concurrent.futures import ThreadPoolExecutor
+    x = np.ascontiguousarray(x, dtype=np.float64)
+    y = np.empty(slabs.n)
+
+    def one(b):
+        spmv_slab_into(*slabs.crs(*b), x, y, b[0])
+
+    with ThreadPoolExecutor(threads or os.cpu_count() or 1) as ex:
+        list(ex.map(one, slabs.bounds))
+    return y
+
+
+def sptrsv_slab(rp, col, val, x, D, b, row_begin, backward=False):
+    """Rows [row_begin, row_begin + m) of o_sptrsv (o_bsptrsv if backward) on the full vectors, in place in x:
+    the strictly triangular slab (rp, col, val) has columns rebased to row_begin.  Forward slabs must run in
+    ascending order, backward ones in descending order, exactly as the whole-matrix loop visits their rows."""
+    lib = load()
+    rb = int(row_begin)
+    (lib.o_bsptrsv if backward else lib.o_sptrsv)(rp.size - 1, rp, col, val, x[rb:], D[rb:], b[rb:])
+
+
+def sptrsv_slabwise(slabs, D, b, backward=False):
+    """x with D x + T x = b for the strictly lower (upper if backward) part T of the slabbed matrix"""
+    x = np.zeros(slabs.n)
+    D = np.ascontiguousarray(D, dtype=np.float64)
+    b = np.ascontiguousarray(b, dtype=np.float64)
+    for rb, re in (reversed(slabs.bounds) if backward else slabs.bounds):
+        L, U, _ = slabs.split(rb, re)
+        sptrsv_slab(*(U if backward else L), x, D, b, rb, backward)
+    return x
+
+
 def _vp(a):
     return None if a is None else a.ctypes.data
 
