@@ -209,6 +209,7 @@ struct bis_context {
                                 // + 1 byte per nonzero of memory; 0 = stream the values; see DESIGN.md 3.1)
     int last_spmv_value_bytes = 8;   // bytes per nonzero the last windowed SpMV streamed for the values (8 or 1)
     int64_t last_spmv_stream_bytes = 0;   // compulsory HBM bytes of the last windowed SpMV launch (its format's byte model)
+    int last_spmv_format = 0;        // tile format of the last windowed SpMV: 3 x windows, 4 grid tiles (WinFormat::grid)
     int opt_wave_cluster = 8;   // stencil wavefront: planes per thread-block cluster (1: no clusters, every hand-over through L2)
     int opt_wave_backoff_ns = 0;      // ... nanoseconds a plane fed through L2 falls back after it had to poll (clusters only)
     int wave_cluster_used = 0;  // ... what the last solve ran with
@@ -325,6 +326,14 @@ struct WinFormat {
     unsigned short *d_seg_off = nullptr;
     int *d_nseg = nullptr;
     unsigned short *d_lidx = nullptr;
+    // grid tiles (bis_spmv_win.cuh): a matrix on its grid hint whose nonzeros all lie in the 27-point stencil of their
+    // row, in ascending order, with at most 256 distinct row patterns, needs neither the window table nor lidx: a tile's
+    // x is one 3-D box of the grid, and a row is described by the 27-bit mask of its stencil cells
+    int grid = 0;                  // 1: this format (seg_* / lidx are not allocated)
+    int gx = 0, gy = 0, gz = 0;    // the grid, x fastest
+    int n_class = 0;
+    unsigned int *d_class_mask = nullptr;   // [256] cell mask of each row class, ascending
+    unsigned char *d_row_class = nullptr;   // [n_rows] class of every row
     // value dictionary (lossless): when the matrix holds at most 256 distinct values (constant-coefficient stencils:
     // HPCG has two), the tiles stream a 1-byte index per nonzero instead of the 8-byte value and the kernel looks the
     // value up in a 2 KB table in shared memory -- the bits of every product are those of the CRS value

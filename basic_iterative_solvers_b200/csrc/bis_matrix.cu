@@ -58,6 +58,8 @@ void free_matrix_storage(bis_matrix *A) {
     cudaFree(A->win.d_order);
     cudaFree(A->win.d_vidx);
     cudaFree(A->win.d_vdict);
+    cudaFree(A->win.d_class_mask);
+    cudaFree(A->win.d_row_class);
 }
 
 template <typename RP>

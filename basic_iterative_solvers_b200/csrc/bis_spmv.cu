@@ -22,6 +22,8 @@
 #include "bis_device.cuh"
 #include "bis_spmv_tma.cuh"
 #include "bis_spmv_win.cuh"
+#include <cudaTypedefs.h>
+
 #include <algorithm>
 #include <cstdio>
 #include <cstdlib>
@@ -339,6 +341,163 @@ int win_free(bis_matrix *A) {
     w.d_seg_start = nullptr; w.d_seg_len = nullptr; w.d_seg_off = nullptr; w.d_nseg = nullptr; w.d_lidx = nullptr;
     w.d_order = nullptr; w.d_vidx = nullptr; w.d_vdict = nullptr;
     w.dict_state = 0; w.n_dict = 0;
+    cudaFree(w.d_class_mask); cudaFree(w.d_row_class);
+    w.d_class_mask = nullptr; w.d_row_class = nullptr;
+    w.grid = 0; w.n_class = 0;
+    return 0;
+}
+
+// ---- grid tiles (WinFormat::grid) ------------------------------------------------------------------
+// A row's cell mask: bit 9 (dz+1) + 3 (dy+1) + (dx+1) for each nonzero at grid offset (dx, dy, dz).  GRID_BAD when a
+// nonzero lies outside the row's 27-point stencil or inside the grid, or the columns do not ascend strictly.  The
+// cells inside the grid have strictly ascending columns, so one forward walk over them matches the row.
+constexpr unsigned int GRID_BAD = 0xFFFFFFFFu;    // also the empty slot of the class table (masks have 27 bits)
+constexpr int GRID_SLOTS = 1024;
+
+template <typename RP>
+__device__ __forceinline__ unsigned int grid_row_mask(uint32_t r, const RP *rp, const int *col, uint32_t nx, uint32_t ny,
+                                                      uint32_t nz) {
+    const int xr = (int)(r % nx), t = (int)(r / nx), yr = t % (int)ny, zr = t / (int)ny;
+    const int plane = (int)(nx * ny);
+    unsigned int m = 0;
+    int j = 0;
+    for (int64_t k = (int64_t)rp[r]; k < (int64_t)rp[r + 1]; ++k) {
+        const int d = col[k] - (int)r;
+        for (;; ++j) {
+            if (j == 27) return GRID_BAD;
+            const int dz = j / 9 - 1, dy = (j / 3) % 3 - 1, dx = j % 3 - 1;
+            if (xr + dx < 0 || xr + dx >= (int)nx || yr + dy < 0 || yr + dy >= (int)ny || zr + dz < 0 || zr + dz >= (int)nz)
+                continue;
+            const int dj = dz * plane + dy * (int)nx + dx;
+            if (dj < d) continue;
+            if (dj > d) return GRID_BAD;
+            break;
+        }
+        m |= 1u << j;
+        ++j;
+    }
+    return m;
+}
+
+// Pass 1: the distinct row masks into a global table (a row inserts only when its mask differs from the previous
+// row's, so interior runs cost one lookup per warp); state[0] counts them, state[1] = 1 means not a grid matrix.
+template <typename RP>
+__global__ void __launch_bounds__(256) grid_collect_kernel(uint32_t n, const RP *rp, const int *col, uint32_t nx, uint32_t ny,
+                                                           uint32_t nz, unsigned int *slots, int *state) {
+    const uint32_t stride = gridDim.x * blockDim.x;
+    for (uint32_t r0 = blockIdx.x * blockDim.x; r0 < n; r0 += stride) {
+        if (*reinterpret_cast<volatile int *>(state + 1)) return;      // warp-uniform: r0 is
+        const uint32_t r = r0 + threadIdx.x;
+        const unsigned int m = r < n ? grid_row_mask(r, rp, col, nx, ny, nz) : 0u;
+        const unsigned int prev = __shfl_up_sync(0xffffffffu, m, 1);
+        if (r >= n || ((threadIdx.x & 31) != 0 && prev == m)) continue;
+        if (m == GRID_BAD) {
+            atomicExch(state + 1, 1);
+            continue;
+        }
+        unsigned int g = (m * 2654435761u) >> 22;     // 10 bits
+        for (int probe = 0; probe < GRID_SLOTS; ++probe, g = (g + 1) & (GRID_SLOTS - 1)) {
+            const unsigned int cur = *reinterpret_cast<volatile unsigned int *>(&slots[g]);
+            if (cur == m) break;
+            if (cur == GRID_BAD) {
+                const unsigned int old = atomicCAS(&slots[g], GRID_BAD, m);
+                if (old == GRID_BAD) {
+                    if (atomicAdd(state, 1) + 1 > 256) atomicExch(state + 1, 1);
+                    break;
+                }
+                if (old == m) break;
+            }
+        }
+    }
+}
+
+// Pass 2: the class of every row (its mask's place in the ascending table)
+template <typename RP>
+__global__ void __launch_bounds__(256) grid_classify_kernel(uint32_t n, const RP *rp, const int *col, uint32_t nx, uint32_t ny,
+                                                            uint32_t nz, const unsigned int *masks, int n_class,
+                                                            unsigned char *cls) {
+    __shared__ unsigned int s_m[256];
+    for (int i = threadIdx.x; i < 256; i += blockDim.x) s_m[i] = i < n_class ? masks[i] : GRID_BAD;
+    __syncthreads();
+    for (uint32_t r = blockIdx.x * blockDim.x + threadIdx.x; r < n; r += gridDim.x * blockDim.x) {
+        const unsigned int m = grid_row_mask(r, rp, col, nx, ny, nz);
+        int lo = 0, hi = n_class - 1;
+        while (lo < hi) {
+            const int mid = (lo + hi) >> 1;
+            if (s_m[mid] < m) lo = mid + 1;
+            else hi = mid;
+        }
+        cls[r] = (unsigned char)lo;
+    }
+}
+
+// Sets w.grid = 1 and builds the row classes when A qualifies for grid tiles of R rows (see WinFormat::grid).
+template <typename RP>
+int grid_build_t(bis_context *c, const bis_matrix *A, int R) {
+    WinFormat &w = A->win;
+    const uint32_t n = (uint32_t)A->n_rows, nx = (uint32_t)A->grid_nx, ny = (uint32_t)A->grid_ny, nz = (uint32_t)A->grid_nz;
+    const RP *rp = static_cast<const RP *>(A->d_rp);
+    unsigned int *d_slots = nullptr;
+    int *d_state = nullptr;
+    BIS_CUDA(bis_cuda_malloc(&d_slots, sizeof(unsigned int) * GRID_SLOTS));
+    BIS_CUDA(bis_cuda_malloc(&d_state, 2 * sizeof(int)));
+    BIS_CUDA(cudaMemsetAsync(d_slots, 0xFF, sizeof(unsigned int) * GRID_SLOTS, c->stream));
+    BIS_CUDA(cudaMemsetAsync(d_state, 0, 2 * sizeof(int), c->stream));
+    const int blocks = bis_blocks_for(A->n_rows, 256, c->sm_count * 8);
+    grid_collect_kernel<RP><<<blocks, 256, 0, c->stream>>>(n, rp, A->d_col, nx, ny, nz, d_slots, d_state);
+    BIS_LAUNCH_CHECK(c);
+    std::vector<unsigned int> slots(GRID_SLOTS);
+    int state[2] = {0, 0};
+    BIS_CUDA(cudaMemcpyAsync(slots.data(), d_slots, sizeof(unsigned int) * GRID_SLOTS, cudaMemcpyDeviceToHost, c->stream));
+    BIS_CUDA(cudaMemcpyAsync(state, d_state, sizeof state, cudaMemcpyDeviceToHost, c->stream));
+    BIS_CUDA(cudaStreamSynchronize(c->stream));
+    cudaFree(d_slots);
+    cudaFree(d_state);
+    std::vector<unsigned int> masks;
+    for (unsigned int m : slots)
+        if (m != GRID_BAD) masks.push_back(m);
+    if (state[1] != 0 || masks.empty() || masks.size() > 256) return 0;
+    std::sort(masks.begin(), masks.end());
+    BIS_CUDA(bis_cuda_malloc(&w.d_class_mask, sizeof(unsigned int) * 256));
+    BIS_CUDA(bis_cuda_malloc(&w.d_row_class, (size_t)A->n_rows));
+    BIS_CUDA(cudaMemcpyAsync(w.d_class_mask, masks.data(), sizeof(unsigned int) * masks.size(), cudaMemcpyHostToDevice, c->stream));
+    grid_classify_kernel<RP><<<blocks, 256, 0, c->stream>>>(n, rp, A->d_col, nx, ny, nz, w.d_class_mask, (int)masks.size(),
+                                                            w.d_row_class);
+    BIS_LAUNCH_CHECK(c);
+    w.n_class = (int)masks.size();
+    w.gx = (int)nx; w.gy = (int)ny; w.gz = (int)nz;
+    w.grid = 1;
+    return 0;
+}
+
+// The hint conditions: one GPU, the grid's point count, tiles that never leave their x line, a box of R + 4 <= 256
+// doubles per line (the tensor copy's limit).  The strides 8 nx and 8 nx ny are then multiples of 16 bytes.
+int grid_build(bis_context *c, const bis_matrix *A, int R) {
+    if (A->distributed || A->grid_nx <= 0 || A->n_cols != A->n_rows || A->row_begin != 0) return 0;
+    if (A->grid_nx * A->grid_ny * A->grid_nz != A->n_rows || A->grid_nx % R != 0 || R + 4 > 256) return 0;
+    return A->rp_bytes == 8 ? grid_build_t<int64_t>(c, A, R) : grid_build_t<int32_t>(c, A, R);
+}
+
+// The x box of grid tiles as a 3-D tensor map over x (nx, ny, nz), box (R + 4, 3, 3); elements outside the grid
+// arrive as zeros.  The driver's encoder is reached through the runtime, so the library links no driver library.
+int encode_x_box(const WinFormat &w, const double *x, CUtensorMap *map) {
+    static PFN_cuTensorMapEncodeTiled_v12000 encode = nullptr;
+    if (!encode) {
+        void *fn = nullptr;
+        cudaDriverEntryPointQueryResult q = cudaDriverEntryPointSymbolNotFound;
+        BIS_CUDA(cudaGetDriverEntryPointByVersion("cuTensorMapEncodeTiled", &fn, 12000, cudaEnableDefault, &q));
+        BIS_REQUIRE(q == cudaDriverEntryPointSuccess && fn, "spmv: the driver has no cuTensorMapEncodeTiled");
+        encode = reinterpret_cast<PFN_cuTensorMapEncodeTiled_v12000>(fn);
+    }
+    const cuuint64_t dims[3] = {(cuuint64_t)w.gx, (cuuint64_t)w.gy, (cuuint64_t)w.gz};
+    const cuuint64_t strides[2] = {(cuuint64_t)w.gx * 8, (cuuint64_t)w.gx * w.gy * 8};
+    const cuuint32_t box[3] = {(cuuint32_t)(w.R + 4), 3, 3};
+    const cuuint32_t estr[3] = {1, 1, 1};
+    const CUresult r = encode(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT64, 3, const_cast<double *>(x), dims, strides, box, estr,
+                              CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    BIS_REQUIRE(r == CUDA_SUCCESS, "spmv: cuTensorMapEncodeTiled failed (%d) for the x box of a %dx%dx%d grid", (int)r, w.gx,
+                w.gy, w.gz);
     return 0;
 }
 
@@ -623,41 +782,47 @@ int win_build(bis_context *c, const bis_matrix *A) {
         while (R > 32 && (size_t)R * A->max_row * 10 > (size_t)40 << 10) R >>= 1;   // ~<= 40 KB of val+lidx per stage
     }
     if ((size_t)R * A->max_row * 10 > (size_t)96 << 10) return 0;                     // rows too long for a tile
-    int sort_cap = 1;
-    while (sort_cap < R * A->max_row) sort_cap <<= 1;
     const int64_t n_tiles = (A->n_rows + R - 1) / R;
-    int *d_status = nullptr;
-    BIS_CUDA(bis_cuda_malloc(&d_status, 2 * sizeof(int)));
-    BIS_CUDA(cudaMemsetAsync(d_status, 0, 2 * sizeof(int), c->stream));
-    BIS_CUDA(bis_cuda_malloc(&w.d_seg_start, sizeof(int) * (size_t)n_tiles * WIN_MAXSEG));
-    BIS_CUDA(bis_cuda_malloc(&w.d_seg_len, sizeof(unsigned short) * (size_t)n_tiles * WIN_MAXSEG));
-    BIS_CUDA(bis_cuda_malloc(&w.d_seg_off, sizeof(unsigned short) * (size_t)n_tiles * WIN_MAXSEG));
-    BIS_CUDA(bis_cuda_malloc(&w.d_nseg, sizeof(int) * (size_t)n_tiles));
-    BIS_CUDA(bis_cuda_malloc(&w.d_lidx, sizeof(unsigned short) * ((size_t)A->nnz + 32)));
-    WinBuildArgs a;
-    a.rp = A->d_rp; a.col = A->d_col; a.n_rows = A->n_rows; a.n_owned = A->n_cols; a.R = R; a.sort_cap = sort_cap;
-    a.seg_start = w.d_seg_start; a.seg_len = w.d_seg_len; a.seg_off = w.d_seg_off; a.nseg = w.d_nseg;
-    a.lidx = w.d_lidx; a.status = d_status;
-    const size_t smem = sizeof(int) * (size_t)sort_cap;
-    if (A->rp_bytes == 8) {
-        BIS_CUDA(cudaFuncSetAttribute(win_build_kernel<int64_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        win_build_kernel<int64_t><<<(unsigned)n_tiles, WIN_BUILD_THREADS, smem, c->stream>>>(a);
-    } else {
-        BIS_CUDA(cudaFuncSetAttribute(win_build_kernel<int32_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        win_build_kernel<int32_t><<<(unsigned)n_tiles, WIN_BUILD_THREADS, smem, c->stream>>>(a);
-    }
-    BIS_LAUNCH_CHECK(c);
-    int status[2] = {0, 0};
-    BIS_CUDA(cudaMemcpyAsync(status, d_status, sizeof status, cudaMemcpyDeviceToHost, c->stream));
-    BIS_CUDA(cudaStreamSynchronize(c->stream));
-    cudaFree(d_status);
-    if (status[1] != 0) {
+    if (grid_build(c, A, R) != 0) {
         win_free(const_cast<bis_matrix *>(A));
-        return 0;
+        return 1;
+    }
+    int status[2] = {0, 0};
+    if (!w.grid) {
+        int sort_cap = 1;
+        while (sort_cap < R * A->max_row) sort_cap <<= 1;
+        int *d_status = nullptr;
+        BIS_CUDA(bis_cuda_malloc(&d_status, 2 * sizeof(int)));
+        BIS_CUDA(cudaMemsetAsync(d_status, 0, 2 * sizeof(int), c->stream));
+        BIS_CUDA(bis_cuda_malloc(&w.d_seg_start, sizeof(int) * (size_t)n_tiles * WIN_MAXSEG));
+        BIS_CUDA(bis_cuda_malloc(&w.d_seg_len, sizeof(unsigned short) * (size_t)n_tiles * WIN_MAXSEG));
+        BIS_CUDA(bis_cuda_malloc(&w.d_seg_off, sizeof(unsigned short) * (size_t)n_tiles * WIN_MAXSEG));
+        BIS_CUDA(bis_cuda_malloc(&w.d_nseg, sizeof(int) * (size_t)n_tiles));
+        BIS_CUDA(bis_cuda_malloc(&w.d_lidx, sizeof(unsigned short) * ((size_t)A->nnz + 32)));
+        WinBuildArgs a;
+        a.rp = A->d_rp; a.col = A->d_col; a.n_rows = A->n_rows; a.n_owned = A->n_cols; a.R = R; a.sort_cap = sort_cap;
+        a.seg_start = w.d_seg_start; a.seg_len = w.d_seg_len; a.seg_off = w.d_seg_off; a.nseg = w.d_nseg;
+        a.lidx = w.d_lidx; a.status = d_status;
+        const size_t smem = sizeof(int) * (size_t)sort_cap;
+        if (A->rp_bytes == 8) {
+            BIS_CUDA(cudaFuncSetAttribute(win_build_kernel<int64_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            win_build_kernel<int64_t><<<(unsigned)n_tiles, WIN_BUILD_THREADS, smem, c->stream>>>(a);
+        } else {
+            BIS_CUDA(cudaFuncSetAttribute(win_build_kernel<int32_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            win_build_kernel<int32_t><<<(unsigned)n_tiles, WIN_BUILD_THREADS, smem, c->stream>>>(a);
+        }
+        BIS_LAUNCH_CHECK(c);
+        BIS_CUDA(cudaMemcpyAsync(status, d_status, sizeof status, cudaMemcpyDeviceToHost, c->stream));
+        BIS_CUDA(cudaStreamSynchronize(c->stream));
+        cudaFree(d_status);
+        if (status[1] != 0) {
+            win_free(const_cast<bis_matrix *>(A));
+            return 0;
+        }
     }
     w.R = R;
     w.cap = (R * A->max_row + 32 + 15) & ~15;      // a tile's nonzeros + the alignment padding of its copies (up to 15 either side)
-    w.xcap = (status[0] + 1) & ~1;
+    w.xcap = w.grid ? 9 * (R + 4) : (status[0] + 1) & ~1;
     if (w.xcap < 2) w.xcap = 2;
     w.n_tiles = n_tiles;
     if (win_build_order(c, A) != 0) {
@@ -678,7 +843,8 @@ struct WinPlan {
 bool win_plan(const bis_context *c, const bis_matrix *A, WinPlan *p) {
     const WinFormat &w = A->win;
     const bool dict = w.dict_state == 1 && c->opt_spmv_vdict;
-    size_t stage = (size_t)w.cap * (dict ? 1 : 8) + (size_t)w.xcap * 8 + (size_t)(w.R + 4) * 8 + (size_t)w.cap * 2;
+    const size_t ids = w.grid ? (size_t)((w.R + 15) & ~15) : (size_t)w.cap * 2;     // row classes or lidx
+    size_t stage = (size_t)w.cap * (dict ? 1 : 8) + (size_t)w.xcap * 8 + (size_t)(w.R + 4) * 8 + ids;
     stage = (stage + 127) & ~(size_t)127;
     const size_t budget = (size_t)(c->opt_spmv_smem_kb > 0 ? c->opt_spmv_smem_kb : 110) << 10;
     int nstage = (int)((budget - 128) / stage);
@@ -704,7 +870,7 @@ bool win_plan(const bis_context *c, const bis_matrix *A, WinPlan *p) {
     p->nstage = nstage;
     p->ngroups = ngroups;
     p->stage_bytes = (int)stage;
-    p->smem_bytes = 128 + stage * nstage;
+    p->smem_bytes = 128 + stage * nstage + (w.grid ? 128 : 0);    // grid tiles: room to put the stages on 128 bytes
     return true;
 }
 
@@ -712,9 +878,17 @@ bool win_plan(const bis_context *c, const bis_matrix *A, WinPlan *p) {
 // publish before the sweep, the senders' flags checked at the first tile that reads ghosts).
 template <typename RP, class Epi, bool FUSED>
 int launch_win(bis_context *c, const bis_matrix *A, const WinPlan &p, const double *x, const Epi &epi, RedArgs &ra) {
-    auto kern = spmv_win_kernel<RP, Epi, FUSED>;
-    BIS_CHECK(bis_ensure_dynamic_smem(c, reinterpret_cast<const void *>(kern), p.smem_bytes));
     const WinFormat &w = A->win;
+    auto kern = spmv_win_kernel<RP, Epi, FUSED, false>;
+    CUtensorMap xmap;
+    memset(&xmap, 0, sizeof xmap);
+    if constexpr (!FUSED) {     // grid tiles are never distributed
+        if (w.grid) {
+            kern = spmv_win_kernel<RP, Epi, false, true>;
+            BIS_CHECK(encode_x_box(w, x, &xmap));
+        }
+    }
+    BIS_CHECK(bis_ensure_dynamic_smem(c, reinterpret_cast<const void *>(kern), p.smem_bytes));
     const int threads = w.R * p.ngroups + 32;         // the consumer groups + the producer warp
     int occ = 1;
     BIS_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, threads, p.smem_bytes));
@@ -727,6 +901,8 @@ int launch_win(bis_context *c, const bis_matrix *A, const WinPlan &p, const doub
     if (grid < 1) grid = 1;
     SpmvWinIn in;
     in.rp = A->d_rp; in.val = A->d_val; in.lidx = w.d_lidx;
+    in.row_class = w.d_row_class; in.class_mask = w.d_class_mask; in.n_class = w.n_class;
+    in.box_w = w.R + 4; in.line_tiles = w.grid ? w.gx / w.R : 0; in.gy = w.gy;
     in.seg_start = w.d_seg_start; in.seg_len = w.d_seg_len; in.seg_off = w.d_seg_off; in.nseg = w.d_nseg;
     in.x = x; in.n_rows = A->n_rows;
     in.ord.order = w.d_order;
@@ -742,10 +918,12 @@ int launch_win(bis_context *c, const bis_matrix *A, const WinPlan &p, const doub
     in.val_region = dict ? w.cap : w.cap * 8;
     in.amask = dict ? 15 : 7;
     c->last_spmv_value_bytes = dict ? 1 : 8;
-    // the launch's compulsory HBM bytes in this format: value (8 B or a 1-byte dictionary index) and 16-bit column id
-    // per nonzero, the row_ptr slices, x once, and the vectors of the epilogue (the x windows are re-read from L2)
-    c->last_spmv_stream_bytes = (int64_t)(dict ? 3 : 10) * A->nnz + (int64_t)A->rp_bytes * (A->n_rows + 1) +
-                                8 * (A->n_cols + (int64_t)epi.vectors(x) * A->n_rows);
+    c->last_spmv_format = w.grid ? 4 : 3;
+    // the launch's compulsory HBM bytes in this format: value (8 B or a 1-byte dictionary index) per nonzero, and the
+    // 16-bit column id per nonzero (windows) or the class byte per row (grid tiles), the row_ptr slices, x once, and
+    // the vectors of the epilogue (the x windows and boxes are re-read from L2)
+    c->last_spmv_stream_bytes = (int64_t)(dict ? 1 : 8) * A->nnz + (w.grid ? A->n_rows : 2 * A->nnz) +
+                                (int64_t)A->rp_bytes * (A->n_rows + 1) + 8 * (A->n_cols + (int64_t)epi.vectors(x) * A->n_rows);
 #ifdef BIS_PERF_DEBUG
     in.debug = c->opt_spmv_debug;
     in.stamps = nullptr;
@@ -776,10 +954,10 @@ int launch_win(bis_context *c, const bis_matrix *A, const WinPlan &p, const doub
         HaloFuse hf;
         BIS_CHECK(bis_halo_fuse_args(c, A, &hf));
         in.ghost = A->halo.cur_ghost;
-        kern<<<(unsigned)grid, threads, p.smem_bytes, c->stream>>>(in, epi, ra, hf);
+        kern<<<(unsigned)grid, threads, p.smem_bytes, c->stream>>>(in, epi, ra, hf, xmap);
     } else {
         in.ghost = A->halo.cur_ghost;
-        kern<<<(unsigned)grid, threads, p.smem_bytes, c->stream>>>(in, epi, ra, NoHaloFuse{});
+        kern<<<(unsigned)grid, threads, p.smem_bytes, c->stream>>>(in, epi, ra, NoHaloFuse{}, xmap);
     }
     BIS_LAUNCH_CHECK(c);
 #ifdef BIS_PERF_DEBUG

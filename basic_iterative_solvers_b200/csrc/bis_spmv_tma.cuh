@@ -26,6 +26,8 @@
 
 #include "bis_device.cuh"
 
+#include <cuda.h>
+
 namespace tma {
 
 __device__ __forceinline__ uint32_t smem_u32(const void *p) {
@@ -72,6 +74,17 @@ __device__ __forceinline__ void bulk_g2s(void *dst, const void *src, uint32_t by
         "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint "
         "[%0], [%1], %2, [%3], %4;" ::"r"(smem_u32(dst)),
         "l"(src), "r"(bytes), "r"(smem_u32(bar)), "l"(policy)
+        : "memory");
+}
+
+// 3-D tensor copy global -> shared of the box at (c0, c1, c2) of `map` (cuTensorMapEncodeTiled); dst 128-byte aligned.
+// Elements outside the tensor arrive as zeros and count towards the transaction bytes like the others.
+__device__ __forceinline__ void tensor3d_g2s(void *dst, const CUtensorMap *map, int c0, int c1, int c2, uint64_t *bar,
+                                             uint64_t policy) {
+    asm volatile(
+        "cp.async.bulk.tensor.3d.shared::cluster.global.tile.mbarrier::complete_tx::bytes.L2::cache_hint "
+        "[%0], [%1, {%2, %3, %4}], [%5], %6;" ::"r"(smem_u32(dst)),
+        "l"(reinterpret_cast<uint64_t>(map)), "r"(c0), "r"(c1), "r"(c2), "r"(smem_u32(bar)), "l"(policy)
         : "memory");
 }
 

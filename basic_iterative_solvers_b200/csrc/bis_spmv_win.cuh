@@ -18,6 +18,13 @@
 // are re-read from L2.  The tile format is an acceleration structure derived from
 // the CRS arrays, which stay resident and authoritative; matrices whose tiles need
 // more than WIN_MAXSEG windows (unstructured sparsity) keep using variant 2.
+//
+// Grid tiles (WinFormat::grid): on a matrix that lives on its grid hint with R | nx, the windows of a 27-point
+// tile are the 3 x 3 lines (z-1..z+1, y-1..y+1) over x in [x0-2, x0+R+2) -- one 3-D box of x, fetched by ONE
+// tensor copy -- and every nonzero of row i sits at box position i + C(cell), cell = (dz, dy, dx) in 0..26.  A
+// row is then fully described by the mask of its cells (columns ascend with the cell, so storage order is cell
+// order): the tile streams one class byte per row (an index into <= 256 masks) instead of a 16-bit id per
+// nonzero, and the producer issues four copies per tile instead of twelve, with no window table to load.
 #pragma once
 
 #include <type_traits>
@@ -310,9 +317,16 @@ struct SpmvWinIn {
     int n_dict;
     int val_region;               // bytes of a stage's value part: cap * 8, or cap with the dictionary
     int amask;                    // copies start at element (rp[r0] & ~amask): 7, or 15 with the dictionary (16-byte units)
+    // grid tiles: the class byte of every row, the class masks, and the box of x (the tensor map is a kernel parameter)
+    const unsigned char *row_class;
+    const unsigned int *class_mask;
+    int n_class;
+    int box_w;                    // x extent of the box: R + 4 (a multiple of 2, so its lines are 16-byte multiples)
+    int line_tiles;               // tiles per x line (nx / R)
+    int gy;
     int R;                        // rows per tile == consumer threads
     int cap;                      // nonzeros per stage (multiple of 16)
-    int xcap;                     // window doubles per stage (even)
+    int xcap;                     // window doubles per stage (even); grid tiles: 9 * box_w
     int nstage;                   // stages of the pipeline (tile s lands in stage s % nstage)
     int ngroups;                  // consumer groups (tile s is computed by group s % ngroups); nstage is a multiple of it
     int stage_bytes;
@@ -345,7 +359,8 @@ enum WinStamp {
     WIN_NSTAMP = 16     // the host writes the launch's grid size into the last slot
 };
 
-// stage layout: [val cap*8 | vidx cap][xwin xcap*8][rp (R+4)*8][lidx cap*2], every part 16-byte aligned
+// stage layout: [xwin xcap*8][val cap*8 | vidx cap][rp (R+4)*8][lidx cap*2 | row classes R], every part 16-byte
+// aligned; stages are 128-byte multiples, so the x box of grid tiles lands on the 128-byte boundary a tensor copy needs
 constexpr int WIN_MAX_THREADS = 544;   // consumer groups (R x nstage <= 512) + the producer warp
 
 // This CTA's sequence of tiles: the s-th one is position pos0[i] + b + (s - cum[i]) * G of slab i.
@@ -376,13 +391,15 @@ struct WinSeq {
     }
 };
 
-template <typename RP, class Epi, bool DIST = false>
+template <typename RP, class Epi, bool DIST = false, bool GRID = false>
 __global__ void __launch_bounds__(WIN_MAX_THREADS, 1)
-spmv_win_kernel(SpmvWinIn in, Epi epi, RedArgs ra, typename std::conditional<DIST, HaloFuse, NoHaloFuse>::type hf) {
+spmv_win_kernel(SpmvWinIn in, Epi epi, RedArgs ra, typename std::conditional<DIST, HaloFuse, NoHaloFuse>::type hf,
+                const __grid_constant__ CUtensorMap xmap) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     uint64_t *full = reinterpret_cast<uint64_t *>(smem_raw);            // [MAX_STAGES]
     uint64_t *empty = full + tma::MAX_STAGES;                           // [MAX_STAGES]
     unsigned char *stages = smem_raw + 128;
+    if constexpr (GRID) stages += (128u - (tma::smem_u32(stages) & 127u)) & 127u;     // the plan reserves these bytes
     const int R = in.R;
     // one consumer GROUP (R threads) per stage: group g computes the tiles that land in stage g, so
     // while one group walks its rows the next tile's group is already waiting on its own barrier and
@@ -403,6 +420,9 @@ spmv_win_kernel(SpmvWinIn in, Epi epi, RedArgs ra, typename std::conditional<DIS
     __shared__ double s_dict[256];
     if (in.vidx)
         for (int i = threadIdx.x; i < in.n_dict; i += blockDim.x) s_dict[i] = in.vdict[i];
+    __shared__ unsigned int s_mask[GRID ? 256 : 1];
+    if constexpr (GRID)
+        for (int i = threadIdx.x; i < in.n_class; i += blockDim.x) s_mask[i] = in.class_mask[i];
     if (threadIdx.x == 0) {
         for (int s = 0; s < in.nstage; ++s) {
             tma::mbar_init(&full[s], 1);
@@ -453,8 +473,9 @@ spmv_win_kernel(SpmvWinIn in, Epi epi, RedArgs ra, typename std::conditional<DIS
         const uint64_t pol_stream = tma::policy_evict_first();
         uint64_t pol_keep;
         asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol_keep));
-        // What this lane copies for one tile: lane 0 val, lane 1 lidx, lane 2 the row_ptr slice,
-        // lanes 3.. one x window each.  Everything the copies are described by comes from global
+        // What this lane copies for one tile: lane 0 val, lane 1 lidx (grid tiles: the row classes), lane 2
+        // the row_ptr slice, lanes 3.. one x window each (grid tiles: lane 3 the x box).  Everything the copies
+        // are described by comes from global
         // memory -- the tile id from the order table, then row_ptr and the window table -- so the
         // tile ids are requested 2*PDEPTH and the descriptors PDEPTH tiles ahead: the producer never
         // sits on a global-load latency between two tiles.
@@ -467,8 +488,8 @@ spmv_win_kernel(SpmvWinIn in, Epi epi, RedArgs ra, typename std::conditional<DIS
             unsigned short len, off; // window length / offset    (lanes 3..)
             int tile;                // raw order entry
         };
-        const uint32_t off_xw = (uint32_t)in.val_region;
-        const uint32_t off_rp = off_xw + (uint32_t)in.xcap * 8u;
+        const uint32_t off_val = (uint32_t)in.xcap * 8u;
+        const uint32_t off_rp = off_val + (uint32_t)in.val_region;
         const uint32_t off_li = off_rp + (uint32_t)(R + 4) * 8u;
         auto tile_rows = [&](int tile, int64_t &r0, int64_t &r1) {
             r0 = (int64_t)tile * R;
@@ -493,7 +514,7 @@ spmv_win_kernel(SpmvWinIn in, Epi epi, RedArgs ra, typename std::conditional<DIS
             if (lane < 2) {
                 d.a = rp[r0];
                 d.b = rp[r1];
-            } else if (lane >= 3 && lane - 3 < WIN_MAXSEG) {
+            } else if (!GRID && lane >= 3 && lane - 3 < WIN_MAXSEG) {
                 const int64_t q = (int64_t)tile * WIN_MAXSEG + (lane - 3);
                 d.start = in.seg_start[q];
                 d.len = in.seg_len[q];
@@ -535,35 +556,59 @@ spmv_win_kernel(SpmvWinIn in, Epi epi, RedArgs ra, typename std::conditional<DIS
             tile_rows(d.tile & ~WIN_ORDER_GHOST, r0, r1);
             const void *src = nullptr;
             uint32_t bytes = 0, dst = 0;
-            if (lane < 2) {
-                const int64_t am = in.amask;
-                const int64_t s_al = (int64_t)d.a & ~am;
-                const uint32_t n_el = (uint32_t)((((int64_t)d.b + am) & ~am) - s_al);
+            uint32_t total = 0;
+            if constexpr (GRID) {
+                // every tile is whole (R | nx): only the value copy varies in size, and lane 0 knows it
                 if (lane == 0) {
-                    if (in.vidx) {
-                        src = in.vidx + s_al;
-                        bytes = n_el;
-                    } else {
-                        src = in.val + s_al;
-                        bytes = n_el * 8u;
-                    }
-                } else {
-                    src = in.lidx + s_al;
-                    bytes = n_el * 2u;
+                    const int64_t am = in.amask;
+                    const int64_t s_al = (int64_t)d.a & ~am;
+                    const uint32_t n_el = (uint32_t)((((int64_t)d.b + am) & ~am) - s_al);
+                    src = in.vidx ? static_cast<const void *>(in.vidx + s_al) : static_cast<const void *>(in.val + s_al);
+                    bytes = in.vidx ? n_el : n_el * 8u;
+                    dst = off_val;
+                    total = bytes + (uint32_t)R + (uint32_t)(((R + 1) + 3) & ~3) * (uint32_t)sizeof(RP) +
+                            (BIS_WIN_DEBUG(in, 2) ? 0u : (uint32_t)in.xcap * 8u);
+                } else if (lane == 1) {
+                    src = in.row_class + r0;
+                    bytes = (uint32_t)R;
                     dst = off_li;
+                } else if (lane == 2) {
+                    src = rp + r0;
+                    bytes = (uint32_t)(((R + 1) + 3) & ~3) * (uint32_t)sizeof(RP);
+                    dst = off_rp;
                 }
-            } else if (lane == 2) {
-                src = rp + r0;
-                bytes = (uint32_t)(((r1 - r0 + 1) + 3) & ~(int64_t)3) * (uint32_t)sizeof(RP);
-                dst = off_rp;
-            } else if (d.len && !BIS_WIN_DEBUG(in, 2)) {
-                src = d.start >= 0 ? in.x + d.start : in.ghost + (~d.start);
-                bytes = (uint32_t)d.len * 8u;
-                dst = off_xw + (uint32_t)d.off * 8u;
-            }
-            uint32_t total = bytes;
+            } else {
+                if (lane < 2) {
+                    const int64_t am = in.amask;
+                    const int64_t s_al = (int64_t)d.a & ~am;
+                    const uint32_t n_el = (uint32_t)((((int64_t)d.b + am) & ~am) - s_al);
+                    if (lane == 0) {
+                        if (in.vidx) {
+                            src = in.vidx + s_al;
+                            bytes = n_el;
+                        } else {
+                            src = in.val + s_al;
+                            bytes = n_el * 8u;
+                        }
+                        dst = off_val;
+                    } else {
+                        src = in.lidx + s_al;
+                        bytes = n_el * 2u;
+                        dst = off_li;
+                    }
+                } else if (lane == 2) {
+                    src = rp + r0;
+                    bytes = (uint32_t)(((r1 - r0 + 1) + 3) & ~(int64_t)3) * (uint32_t)sizeof(RP);
+                    dst = off_rp;
+                } else if (d.len && !BIS_WIN_DEBUG(in, 2)) {
+                    src = d.start >= 0 ? in.x + d.start : in.ghost + (~d.start);
+                    bytes = (uint32_t)d.len * 8u;
+                    dst = (uint32_t)d.off * 8u;
+                }
+                total = bytes;
 #pragma unroll
-            for (int o = 16; o > 0; o >>= 1) total += __shfl_xor_sync(0xffffffffu, total, o);
+                for (int o = 16; o > 0; o >>= 1) total += __shfl_xor_sync(0xffffffffu, total, o);
+            }
 #ifdef BIS_PERF_DEBUG
             const long long t_w0 = clock64();
 #endif
@@ -577,6 +622,15 @@ spmv_win_kernel(SpmvWinIn in, Epi epi, RedArgs ra, typename std::conditional<DIS
             if (lane == 0) tma::mbar_expect_tx(&full[st], total);
             __syncwarp();
             if (bytes) tma::bulk_g2s(sb + dst, src, bytes, &full[st], lane < 3 ? pol_stream : pol_keep);
+            if constexpr (GRID) {
+                if (lane == 3 && !BIS_WIN_DEBUG(in, 2)) {
+                    // box origin (x0 - 2, y - 1, z - 1): x0 - 2 keeps the box lines on 16-byte boundaries of x
+                    const int line = (d.tile & ~WIN_ORDER_GHOST) / in.line_tiles;
+                    const int x0 = ((d.tile & ~WIN_ORDER_GHOST) - line * in.line_tiles) * R;
+                    const int z = line / in.gy;
+                    tma::tensor3d_g2s(sb, &xmap, x0 - 2, line - z * in.gy - 1, z - 1, &full[st], pol_keep);
+                }
+            }
 #ifdef BIS_PERF_DEBUG
             __syncwarp();
             pst[WS_P_EMPTY] += t_w1 - t_w0;
@@ -668,10 +722,10 @@ spmv_win_kernel(SpmvWinIn in, Epi epi, RedArgs ra, typename std::conditional<DIS
             if (s + in.ngroups < my_tiles) raw_next = in.ord.order[seq.pos(in.ord, (int)blockIdx.x, s + in.ngroups)];
             const int64_t row = (int64_t)tile * R + tid_g;
             const unsigned char *sb = stages + (size_t)st * in.stage_bytes;
-            const double *__restrict__ sval = reinterpret_cast<const double *>(sb);
-            const unsigned char *__restrict__ svi = sb;
-            const double *__restrict__ sxw = reinterpret_cast<const double *>(sb + in.val_region);
-            const RP *__restrict__ srp = reinterpret_cast<const RP *>(sxw + in.xcap);
+            const double *__restrict__ sxw = reinterpret_cast<const double *>(sb);
+            const double *__restrict__ sval = sxw + in.xcap;
+            const unsigned char *__restrict__ svi = reinterpret_cast<const unsigned char *>(sval);
+            const RP *__restrict__ srp = reinterpret_cast<const RP *>(svi + in.val_region);
             const unsigned short *__restrict__ sli =
                 reinterpret_cast<const unsigned short *>(reinterpret_cast<const unsigned char *>(srp) + (size_t)(R + 4) * 8);
             EpiPre pre{0.0, 0.0, 0.0};
@@ -700,30 +754,73 @@ spmv_win_kernel(SpmvWinIn in, Epi epi, RedArgs ra, typename std::conditional<DIS
                 const int ke = (int)((int64_t)srp[tid_g + 1] - base);
                 double sum = 0.0;
                 int k = ks;
-                if (in.vidx) {          // the same walk with the value looked up by its 1-byte index (warp-uniform)
+                if constexpr (GRID) {
+                    // the row's nonzeros in storage order are the set bits of its cell mask in ascending order;
+                    // cell c = 9 (dz+1) + 3 (dy+1) + (dx+1) reads box position row + (c / 3) * box_w + c % 3 + 1
+                    unsigned int m = s_mask[reinterpret_cast<const unsigned char *>(sli)[tid_g]];
+                    const double *__restrict__ xr = sxw + tid_g + 1;
+                    const int w3 = in.box_w - 3;
+                    auto next_x = [&]() {
+                        const unsigned int c = (unsigned int)__ffs((int)m) - 1u;
+                        m &= m - 1u;
+                        return xr[(int)(c / 3u) * w3 + (int)c];
+                    };
+                    if (in.vidx) {
+                        for (; k + 9 <= ke; k += 9) {
+                            double a[9], xv[9];
+#pragma unroll
+                            for (int u = 0; u < 9; ++u) {
+                                a[u] = s_dict[svi[k + u]];
+                                xv[u] = next_x();
+                            }
+#pragma unroll
+                            for (int u = 0; u < 9; ++u) sum = add_rn(sum, mul_rn(a[u], xv[u]));
+                        }
+                        for (; k < ke; ++k) {
+                            const double xv = next_x();
+                            sum = add_rn(sum, mul_rn(s_dict[svi[k]], xv));
+                        }
+                    }
                     for (; k + 9 <= ke; k += 9) {
                         double a[9], xv[9];
 #pragma unroll
                         for (int u = 0; u < 9; ++u) {
-                            a[u] = s_dict[svi[k + u]];
+                            a[u] = sval[k + u];
+                            xv[u] = next_x();
+                        }
+#pragma unroll
+                        for (int u = 0; u < 9; ++u) sum = add_rn(sum, mul_rn(a[u], xv[u]));
+                    }
+                    for (; k < ke; ++k) {
+                        const double xv = next_x();
+                        sum = add_rn(sum, mul_rn(sval[k], xv));
+                    }
+                } else {
+                    if (in.vidx) {          // the same walk with the value looked up by its 1-byte index (warp-uniform)
+                        for (; k + 9 <= ke; k += 9) {
+                            double a[9], xv[9];
+#pragma unroll
+                            for (int u = 0; u < 9; ++u) {
+                                a[u] = s_dict[svi[k + u]];
+                                xv[u] = sxw[sli[k + u]];
+                            }
+#pragma unroll
+                            for (int u = 0; u < 9; ++u) sum = add_rn(sum, mul_rn(a[u], xv[u]));
+                        }
+                        for (; k < ke; ++k) sum = add_rn(sum, mul_rn(s_dict[svi[k]], sxw[sli[k]]));
+                    }
+                    for (; k + 9 <= ke; k += 9) {
+                        double a[9], xv[9];
+#pragma unroll
+                        for (int u = 0; u < 9; ++u) {
+                            a[u] = sval[k + u];
                             xv[u] = sxw[sli[k + u]];
                         }
 #pragma unroll
                         for (int u = 0; u < 9; ++u) sum = add_rn(sum, mul_rn(a[u], xv[u]));
                     }
-                    for (; k < ke; ++k) sum = add_rn(sum, mul_rn(s_dict[svi[k]], sxw[sli[k]]));
+                    for (; k < ke; ++k) sum = add_rn(sum, mul_rn(sval[k], sxw[sli[k]]));
                 }
-                for (; k + 9 <= ke; k += 9) {
-                    double a[9], xv[9];
-#pragma unroll
-                    for (int u = 0; u < 9; ++u) {
-                        a[u] = sval[k + u];
-                        xv[u] = sxw[sli[k + u]];
-                    }
-#pragma unroll
-                    for (int u = 0; u < 9; ++u) sum = add_rn(sum, mul_rn(a[u], xv[u]));
-                }
-                for (; k < ke; ++k) sum = add_rn(sum, mul_rn(sval[k], sxw[sli[k]]));
                 epi(row, sum, pre, acc);
             }
             __syncwarp();

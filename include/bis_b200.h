@@ -105,7 +105,8 @@ int bis_flush_l2(bis_context *ctx);
  * index per nonzero instead of the 8-byte value -- lossless, same bits, + 1 byte
  * per nonzero of memory; 0: the values are streamed;
  * "spmv_value_bytes" reads back what the last launch streamed, "spmv_stream_mb" its
- * compulsory HBM bytes in units of 1e6 from the format's byte model), "wave_cluster" (stencil
+ * compulsory HBM bytes in units of 1e6 from the format's byte model, "spmv_format"
+ * its tile format: 3 x windows, 4 grid tiles), "wave_cluster" (stencil
  * wavefront: planes per thread-block cluster, 1 / 2 / 4 / 8 (default) / 16;
  * 1 = every plane-to-plane hand-over through L2), "perm_mode" (0 none,
  * 1 multicolouring, 2 BFS levels, 3 reverse Cuthill-McKee, 4 Cuthill-McKee:
