@@ -123,6 +123,12 @@ _SIGS = {
     "bis_block_cg_update": ([c_ctx, cint, i64, cint] + [c_dev] * 5 + [cint] * 4 + [c_dev], cint),
     "bis_block_cg_direction_x": ([c_ctx, i64, cint] + [c_dev] * 5 + [cint] * 3 + [c_dev], cint),
     "bis_block_cg_status": ([c_ctx, cint, cint, cint, c_dev], cint),
+    "bis_block_gmres_precond_dot": ([c_ctx, cint, i64, cint] + [c_dev] * 5, cint),
+    "bis_block_mgs_step": ([c_ctx, i64, cint] + [c_dev] * 4 + [cint, c_dev], cint),
+    "bis_block_scale_inv_norm": ([c_ctx, i64, cint] + [c_dev] * 3 + [cint, c_dev], cint),
+    "bis_block_gmres_update_x": ([c_ctx, i64, cint, cint, c_dev, i64, C.c_void_p, c_dev, c_dev, C.c_void_p], cint),
+    "bis_vector_read_begin": ([c_ctx, c_dev, i64], cint),
+    "bis_vector_read_end": ([c_ctx, C.c_void_p, i64], cint),
 }
 
 _lib = None

@@ -14,6 +14,11 @@
 // thread t adds rows t, t+256, t+512, t+768 of each 1024-row trip in that order with fma, then the same warp
 // and block shuffle trees, the same per-slab sums and combine_records.  Only the loads differ (a thread reads
 // the k contiguous values of its row).
+//
+// The GMRES kernels (OP_PDOT, OP_MGS, OP_SCALE, block_update_x_kernel) batch bis_apply_preconditioner(JACOBI) +
+// bis_dot_to_slot, bis_mgs_step, bis_scale_inv_norm and bis_gmres_update_x the same way.  They read their
+// coefficients from, and reduce into, a caller-owned Hessenberg array H ((m+2) x k, entry (l, j) at H[l*k + j])
+// instead of the scalar slots: (m+2) k reaches 1056 values.
 #include "bis_device.cuh"
 #include "bis_spmv_tma.cuh"
 
@@ -281,10 +286,11 @@ int launch_spmm(bis_context *c, const bis_matrix *A, const double *X, double *Y)
 }
 
 // ---- batched streaming kernels -------------------------------------------------------------------------
-enum BlockOp { OP_DOT = 0, OP_RESID = 1, OP_UPDATE = 2, OP_DIRX = 3 };
+enum BlockOp { OP_DOT = 0, OP_RESID = 1, OP_UPDATE = 2, OP_DIRX = 3, OP_PDOT = 4, OP_MGS = 5, OP_SCALE = 6 };
 
 template <int K, int OP> struct BlockNq {
-    static constexpr int value = OP == OP_DOT ? K : (OP == OP_DIRX ? 0 : 2 * K);
+    static constexpr int value = (OP == OP_DOT || OP == OP_PDOT || OP == OP_MGS) ? K
+                               : ((OP == OP_DIRX || OP == OP_SCALE) ? 0 : 2 * K);
 };
 
 struct BlockArgs {
@@ -294,11 +300,12 @@ struct BlockArgs {
     const double *in0, *in1, *in2;   // per OP, see the kernel
     const double *D;                 // [n] diagonal (Jacobi)
     double *out0, *out1, *out2;
-    const double *S;                 // device scalars
-    int slot_a, slot_b, slot_c;      // scalar slot ranges read by the prologue
-    const double *state;             // [3k] block-CG state (thresholds, active flags, iterations) or NULL: all active
+    const double *S;                 // coefficients read by the prologue: the device scalars, or a GMRES H
+    int slot_a, slot_b, slot_c;      // index ranges of S read by the prologue
+    const double *active;            // [k] active flags (0.0: frozen) or NULL: all active
+    double *red_out;                 // where reduced quantities go: the device scalars, or a GMRES H
     double *partials;                // [2*KMAX][BIS_MAX_RED_BLOCKS]
-    int slot_q[BQ_MAX];              // target slot of every reduced quantity (-1: not written)
+    int slot_q[BQ_MAX];              // index in red_out of every reduced quantity (-1: not written)
 };
 
 // Sum of NQ quantities over the grid.  Every step is that of block_reduce_finish / grid_reduce_finish (bis_device.cuh)
@@ -370,7 +377,7 @@ __device__ __forceinline__ void block_reduce_multi(double (&acc)[NQ > 0 ? NQ : 1
             for (int i = 0; i < BIS_NSLAB; ++i)
                 if (i < ra.n_rec) t += r[i];
         }
-        if (a.slot_q[q] >= 0 && s_act[q % K]) ra.scalars[a.slot_q[q]] = t;
+        if (a.slot_q[q] >= 0 && s_act[q % K]) a.red_out[a.slot_q[q]] = t;
     }
     __syncthreads();
     if (threadIdx.x == 0) *ra.counter = 0u;
@@ -385,6 +392,12 @@ __device__ __forceinline__ void block_reduce_multi(double (&acc)[NQ > 0 ? NQ : 1
 //            acc[j] += r*r, acc[K+j] += r*z
 //  OP_DIRX   in0 = Z_new, in1 = P_old, in2 = X_old -> out0 = P_new, out1 = X_new       (bis_cg_direction_x)
 //            a column that is not active carries X_old into X_new and leaves P_new alone
+//  OP_PDOT   in0 = W, in1 = V0 or NULL -> out0 = W      w = w / (1.0*D) (jacobi) ;
+//            acc[j] += w*v0, or w*w without V0          (bis_apply_preconditioner(JACOBI) + bis_dot_to_slot)
+//  OP_MGS    in0 = W, in1 = V_l, in2 = V_next or NULL -> out0 = W
+//            t = w - h*v_l (one fma, h = S[slot_a + j]); acc[j] += t*v_next, or t*t         (bis_mgs_step)
+//  OP_SCALE  in0 = W -> out0 = w * (1.0 / sqrt(S[slot_a + j]))                            (bis_scale_inv_norm)
+//            a column that is not active has none of its outputs written
 template <int K, int OP>
 __global__ void __launch_bounds__(BW_THREADS, 1) block_ew_kernel(BlockArgs a, RedArgs ra) {
     constexpr int NQ = BlockNq<K, OP>::value;
@@ -392,7 +405,9 @@ __global__ void __launch_bounds__(BW_THREADS, 1) block_ew_kernel(BlockArgs a, Re
     __shared__ bool s_act[K];
     if ((int)threadIdx.x < K) {
         const int j = threadIdx.x;
-        s_act[j] = a.state == nullptr || a.state[K + j] != 0.0;
+        s_act[j] = a.active == nullptr || a.active[j] != 0.0;
+        if (OP == OP_MGS) s_c0[j] = a.S[a.slot_a + j];                                          // h_lj
+        if (OP == OP_SCALE) s_c0[j] = div_rn(1.0, sqrt(a.S[a.slot_a + j]));                     // 1 / ||w||
         if (OP == OP_UPDATE) s_c0[j] = div_rn(a.S[a.slot_a + j], a.S[a.slot_b + j]);            // alpha = rz / pAp
         if (OP == OP_DIRX) {
             s_c0[j] = div_rn(a.S[a.slot_b + j], a.S[a.slot_c + j]);                            // alpha = rz / pAp
@@ -450,6 +465,34 @@ __global__ void __launch_bounds__(BW_THREADS, 1) block_ew_kernel(BlockArgs a, Re
                     acc[j] = fma(r, r, acc[j]);
                     acc[K + j] = fma(r, z, acc[K + j]);
                 }
+            } else if constexpr (OP == OP_PDOT) {
+                double w[K], v[K];
+#pragma unroll
+                for (int j = 0; j < K; ++j) { w[j] = a.in0[o + j]; v[j] = a.in1 ? a.in1[o + j] : 0.0; }
+                const double d = a.jacobi ? a.D[i] : 1.0;
+#pragma unroll
+                for (int j = 0; j < K; ++j) {
+                    const double z = a.jacobi ? div_rn(w[j], mul_rn(1.0, d)) : w[j];
+                    if (a.jacobi && s_act[j]) a.out0[o + j] = z;
+                    acc[j] = fma(z, a.in1 ? v[j] : z, acc[j]);
+                }
+            } else if constexpr (OP == OP_MGS) {
+                double w[K], vl[K], vn[K];
+#pragma unroll
+                for (int j = 0; j < K; ++j) { w[j] = a.in0[o + j]; vl[j] = a.in1[o + j]; vn[j] = a.in2 ? a.in2[o + j] : 0.0; }
+#pragma unroll
+                for (int j = 0; j < K; ++j) {
+                    const double t = fma(-s_c0[j], vl[j], w[j]);
+                    if (s_act[j]) a.out0[o + j] = t;
+                    acc[j] = fma(t, a.in2 ? vn[j] : t, acc[j]);
+                }
+            } else if constexpr (OP == OP_SCALE) {
+                double w[K];
+#pragma unroll
+                for (int j = 0; j < K; ++j) w[j] = a.in0[o + j];
+#pragma unroll
+                for (int j = 0; j < K; ++j)
+                    if (s_act[j]) a.out0[o + j] = mul_rn(w[j], s_c0[j]);
             } else {
                 double z[K], p[K], x[K];
 #pragma unroll
@@ -483,6 +526,42 @@ __global__ void block_cg_status_kernel(int k, const double *S, int slot_rr, int 
     if (active && it >= (double)max_iters) active = false;
     if (active) state[2 * k + j] = it + 1.0;
     else state[k + j] = 0.0;
+}
+
+// get_explicit_x's product per column j in mask (bis_gmres_update_x): t = sum_{l<nb} V_l[i,j] y_j[l] added left
+// to right, each product rounded; X = X_old + t.  A thread owns one row; X may be X_old (in place).
+struct BlockY {
+    double y[KMAX * BIS_BLOCK_GMRES_MAX_M];   // y_j[l] at y[j * BIS_BLOCK_GMRES_MAX_M + l]
+};
+template <int K>
+__global__ void __launch_bounds__(256) block_update_x_kernel(int64_t n, int nb, const double *V, int64_t ldv, BlockY y,
+                                                             unsigned mask, double *X, const double *X_old) {
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+        double t[K];
+#pragma unroll
+        for (int j = 0; j < K; ++j) t[j] = 0.0;
+#pragma unroll 1
+        for (int l = 0; l < nb; ++l) {
+            const double *v = V + l * ldv + i * K;
+#pragma unroll
+            for (int j = 0; j < K; ++j) t[j] = add_rn(t[j], mul_rn(v[j], y.y[j * BIS_BLOCK_GMRES_MAX_M + l]));
+        }
+#pragma unroll
+        for (int j = 0; j < K; ++j)
+            if (mask >> j & 1u) X[i * K + j] = add_rn(X_old[i * K + j], t[j]);
+    }
+}
+
+template <int K>
+int launch_update_x_k(bis_context *c, int64_t n, int nb, const double *V, int64_t ldv, const BlockY &y, unsigned mask,
+                      double *X, const double *X_old) {
+    const int blocks = bis_blocks_for(n, 256, c->sm_count * 8);
+    BIS_CHECK(bis_prof_begin(c, BIS_PROF_VECTOR));
+    block_update_x_kernel<K><<<blocks, 256, 0, c->stream>>>(n, nb, V, ldv, y, mask, X, X_old);
+    BIS_LAUNCH_CHECK(c);
+    BIS_CHECK(bis_prof_end(c, BIS_PROF_VECTOR));
+    return 0;
 }
 
 int ensure_block_partials(bis_context *c) {
@@ -561,6 +640,7 @@ BlockArgs block_args(bis_context *c, int64_t n) {
     memset(&a, 0, sizeof a);
     a.n = n;
     a.S = c->d_scalars;
+    a.red_out = c->d_scalars;
     for (int q = 0; q < BQ_MAX; ++q) a.slot_q[q] = -1;
     return a;
 }
@@ -602,7 +682,7 @@ extern "C" int bis_block_dot_to_slots(bis_context *c, int64_t n, int k, const do
     REQ_BLOCK_VEC(B, "B");
     REQ_SLOTS(slot0, k, "slot0");
     BlockArgs a = block_args(c, n);
-    a.in0 = A; a.in1 = B; a.state = state;
+    a.in0 = A; a.in1 = B; a.active = state ? state + k : nullptr;
     for (int j = 0; j < k; ++j) a.slot_q[j] = slot0 + j;
     return launch_block<OP_DOT>(c, k, a);
 }
@@ -638,7 +718,7 @@ extern "C" int bis_block_cg_update(bis_context *c, int precond, int64_t n, int k
     REQ_SLOTS(slot_rz_new0, k, "rz_new");
     BlockArgs a = block_args(c, n);
     a.jacobi = precond == BIS_PRECOND_JACOBI;
-    a.in0 = R_old; a.in1 = AP; a.D = A_D; a.out0 = R_new; a.out1 = Z_new; a.state = state;
+    a.in0 = R_old; a.in1 = AP; a.D = A_D; a.out0 = R_new; a.out1 = Z_new; a.active = state ? state + k : nullptr;
     a.slot_a = slot_rz0; a.slot_b = slot_pAp0;
     for (int j = 0; j < k; ++j) {
         a.slot_q[j] = slot_rr0 + j;
@@ -655,7 +735,7 @@ extern "C" int bis_block_cg_direction_x(bis_context *c, int64_t n, int k, double
     REQ_BLOCK_VEC(X_new, "X_new"); REQ_BLOCK_VEC(X_old, "X_old");
     REQ_SLOTS(slot_rz_new0, k, "rz_new"); REQ_SLOTS(slot_rz0, k, "rz"); REQ_SLOTS(slot_pAp0, k, "pAp");
     BlockArgs a = block_args(c, n);
-    a.in0 = Z_new; a.in1 = P_old; a.in2 = X_old; a.out0 = P_new; a.out1 = X_new; a.state = state;
+    a.in0 = Z_new; a.in1 = P_old; a.in2 = X_old; a.out0 = P_new; a.out1 = X_new; a.active = state ? state + k : nullptr;
     a.slot_a = slot_rz_new0; a.slot_b = slot_rz0; a.slot_c = slot_pAp0;
     return launch_block<OP_DIRX>(c, k, a);
 }
@@ -668,4 +748,82 @@ extern "C" int bis_block_cg_status(bis_context *c, int k, int slot_rr0, int max_
     block_cg_status_kernel<<<1, 32, 0, c->stream>>>(k, c->d_scalars, slot_rr0, max_iters, state);
     BIS_LAUNCH_CHECK(c);
     return 0;
+}
+
+// ---- block GMRES -------------------------------------------------------------------------------------------
+#define REQ_H_ROW(l, lo, hi, what) \
+    BIS_REQUIRE((l) >= (lo) && (l) <= (hi), "%s: l = %d outside [%d, %d]", what, (l), (lo), (hi))
+
+extern "C" int bis_block_gmres_precond_dot(bis_context *c, int precond, int64_t n, int k, double *W, const double *A_D,
+                                           const double *V0, double *H, const double *active) {
+    REQ_BLOCK(c, k);
+    BIS_REQUIRE(precond == BIS_PRECOND_NONE || precond == BIS_PRECOND_JACOBI,
+                "bis_block_gmres_precond_dot: preconditioner %d not supported (none or jacobi)", precond);
+    REQ_BLOCK_VEC(W, "W");
+    BIS_REQUIRE(V0 == nullptr || aligned16(V0), "bis_block_gmres_precond_dot: V0 not 16-byte aligned");
+    BIS_REQUIRE(precond != BIS_PRECOND_JACOBI || A_D, "bis_block_gmres_precond_dot: jacobi needs A_D");
+    BIS_REQUIRE(H, "bis_block_gmres_precond_dot: null H");
+    BlockArgs a = block_args(c, n);
+    a.jacobi = precond == BIS_PRECOND_JACOBI;
+    a.in0 = W; a.in1 = V0; a.D = A_D; a.out0 = W; a.active = active; a.red_out = H;
+    for (int j = 0; j < k; ++j) a.slot_q[j] = j;
+    return launch_block<OP_PDOT>(c, k, a);
+}
+
+extern "C" int bis_block_mgs_step(bis_context *c, int64_t n, int k, double *W, const double *V_l, const double *V_next,
+                                  double *H, int l, const double *active) {
+    REQ_BLOCK(c, k);
+    REQ_BLOCK_VEC(W, "W");
+    REQ_BLOCK_VEC(V_l, "V_l");
+    BIS_REQUIRE(V_next == nullptr || aligned16(V_next), "bis_block_mgs_step: V_next not 16-byte aligned");
+    BIS_REQUIRE(H, "bis_block_mgs_step: null H");
+    REQ_H_ROW(l, 0, BIS_BLOCK_GMRES_MAX_M - 1, "bis_block_mgs_step");
+    BlockArgs a = block_args(c, n);
+    a.in0 = W; a.in1 = V_l; a.in2 = V_next; a.out0 = W; a.active = active;
+    a.S = H; a.slot_a = l * k;
+    a.red_out = H;
+    for (int j = 0; j < k; ++j) a.slot_q[j] = (l + 1) * k + j;
+    return launch_block<OP_MGS>(c, k, a);
+}
+
+extern "C" int bis_block_scale_inv_norm(bis_context *c, int64_t n, int k, double *out, const double *W, const double *H,
+                                        int l, const double *active) {
+    REQ_BLOCK(c, k);
+    REQ_BLOCK_VEC(out, "out");
+    REQ_BLOCK_VEC(W, "W");
+    BIS_REQUIRE(H, "bis_block_scale_inv_norm: null H");
+    REQ_H_ROW(l, 0, BIS_BLOCK_GMRES_MAX_M, "bis_block_scale_inv_norm");
+    BlockArgs a = block_args(c, n);
+    a.in0 = W; a.out0 = out; a.active = active;
+    a.S = H; a.slot_a = l * k;
+    return launch_block<OP_SCALE>(c, k, a);
+}
+
+extern "C" int bis_block_gmres_update_x(bis_context *c, int64_t n, int k, int nb, const double *V, int64_t ldv,
+                                        const double *Y, double *X, const double *X_old, const int *mask) {
+    REQ_BLOCK(c, k);
+    BIS_REQUIRE(nb >= 0 && nb <= BIS_BLOCK_GMRES_MAX_M, "bis_block_gmres_update_x: nb = %d outside [0, %d]", nb,
+                BIS_BLOCK_GMRES_MAX_M);
+    BIS_REQUIRE(nb == 0 || (Y && aligned16(V)), "bis_block_gmres_update_x: null Y, or V null or not 16-byte aligned");
+    BIS_REQUIRE(ldv >= n * k && ldv % 2 == 0, "bis_block_gmres_update_x: ldv = %lld must be even and >= n*k = %lld",
+                (long long)ldv, (long long)(n * k));
+    REQ_BLOCK_VEC(X, "X");
+    REQ_BLOCK_VEC(X_old, "X_old");
+    BIS_REQUIRE(mask, "bis_block_gmres_update_x: null mask");
+    BlockY y;   // copied into the launch's parameters: no host pointer outlives the call
+    memset(&y, 0, sizeof y);
+    unsigned bits = 0;
+    for (int j = 0; j < k; ++j) {
+        if (mask[j]) bits |= 1u << j;
+        for (int l = 0; l < nb; ++l) y.y[j * BIS_BLOCK_GMRES_MAX_M + l] = Y[(size_t)j * nb + l];
+    }
+    if (bits == 0) return 0;
+    switch (k) {
+#define BIS_UPX_CASE(K) case K: return launch_update_x_k<K>(c, n, nb, V, ldv, y, bits, X, X_old);
+    BIS_UPX_CASE(1) BIS_UPX_CASE(2) BIS_UPX_CASE(3) BIS_UPX_CASE(4) BIS_UPX_CASE(5) BIS_UPX_CASE(6)
+    BIS_UPX_CASE(7) BIS_UPX_CASE(8) BIS_UPX_CASE(9) BIS_UPX_CASE(10) BIS_UPX_CASE(11) BIS_UPX_CASE(12)
+    BIS_UPX_CASE(13) BIS_UPX_CASE(14) BIS_UPX_CASE(15) BIS_UPX_CASE(16)
+#undef BIS_UPX_CASE
+    }
+    return 2;
 }

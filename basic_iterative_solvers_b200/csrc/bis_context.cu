@@ -73,6 +73,8 @@ static int context_init(bis_context *c, int device) {
     BIS_CUDA(bis_cuda_malloc(&c->d_scalars, sizeof(double) * BIS_NUM_SCALARS));
     BIS_CUDA(cudaMemset(c->d_scalars, 0, sizeof(double) * BIS_NUM_SCALARS));
     BIS_CUDA(cudaMallocHost(&c->h_scalars, sizeof(double) * BIS_NUM_SCALARS));
+    BIS_CUDA(cudaMallocHost(&c->h_vec_read, sizeof(double) * BIS_VECTOR_READ_MAX));
+    BIS_CUDA(cudaEventCreateWithFlags(&c->ev_vec_read, cudaEventDisableTiming));
     BIS_CUDA(bis_cuda_malloc(&c->d_partials, sizeof(double) * BIS_MAX_RED * BIS_MAX_RED_BLOCKS));
     BIS_CUDA(bis_cuda_malloc(&c->d_counter, sizeof(unsigned int)));
     BIS_CUDA(cudaMemset(c->d_counter, 0, sizeof(unsigned int)));
@@ -178,6 +180,7 @@ extern "C" int bis_context_destroy(bis_context *c) {
     if (c->comm) ncclCommDestroy(c->comm);
     cudaFree(c->d_scalars);
     cudaFreeHost(c->h_scalars);
+    cudaFreeHost(c->h_vec_read);
     cudaFree(c->d_partials);
     cudaFree(c->d_block_partials);
     cudaFree(c->d_counter);
@@ -191,6 +194,7 @@ extern "C" int bis_context_destroy(bis_context *c) {
     cudaEventDestroy(c->ev_main);
     cudaEventDestroy(c->ev_comm);
     cudaEventDestroy(c->ev_scalar);
+    cudaEventDestroy(c->ev_vec_read);
     cudaStreamDestroy(c->stream);
     cudaStreamDestroy(c->comm_stream);
     delete c;
@@ -596,6 +600,24 @@ extern "C" int bis_scalar_read_end(bis_context *c, int first_slot, int count, do
                 "bis_scalar_read_end: bad range [%d,+%d)", first_slot, count);
     BIS_CUDA(cudaEventSynchronize(c->ev_scalar));
     memcpy(values, c->h_scalars + first_slot, sizeof(double) * count);
+    return 0;
+}
+
+// The same split read for a range of device memory (a block GMRES's Hessenberg column), through its own
+// staging buffer and event: it may be outstanding together with one scalar read.
+extern "C" int bis_vector_read_begin(bis_context *c, const double *src, int64_t count) {
+    BIS_REQUIRE(c && src && count > 0 && count <= BIS_VECTOR_READ_MAX,
+                "bis_vector_read_begin: null source or count %lld outside [1, %d]", (long long)count, BIS_VECTOR_READ_MAX);
+    BIS_CUDA(cudaMemcpyAsync(c->h_vec_read, src, sizeof(double) * (size_t)count, cudaMemcpyDeviceToHost, c->stream));
+    BIS_CUDA(cudaEventRecord(c->ev_vec_read, c->stream));
+    return 0;
+}
+
+extern "C" int bis_vector_read_end(bis_context *c, double *dst, int64_t count) {
+    BIS_REQUIRE(c && dst && count > 0 && count <= BIS_VECTOR_READ_MAX,
+                "bis_vector_read_end: null destination or count %lld outside [1, %d]", (long long)count, BIS_VECTOR_READ_MAX);
+    BIS_CUDA(cudaEventSynchronize(c->ev_vec_read));
+    memcpy(dst, c->h_vec_read, sizeof(double) * (size_t)count);
     return 0;
 }
 

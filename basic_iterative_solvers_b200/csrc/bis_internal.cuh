@@ -155,6 +155,8 @@ struct bis_context {
     cudaEvent_t ev_main = nullptr, ev_comm = nullptr, ev_scalar = nullptr;
     double *d_scalars = nullptr;         // BIS_NUM_SCALARS
     double *h_scalars = nullptr;         // pinned staging
+    double *h_vec_read = nullptr;        // [BIS_VECTOR_READ_MAX] pinned staging of bis_vector_read_begin / _end
+    cudaEvent_t ev_vec_read = nullptr;
     double *d_partials = nullptr;
     double *d_block_partials = nullptr;  // [2*BIS_BLOCK_MAX_K][BIS_MAX_RED_BLOCKS]: multi-RHS reductions (bis_block.cu), on first use
     unsigned int *d_counter = nullptr;

@@ -44,10 +44,14 @@ def load() -> C.CDLL:
     lib.bis_host_gmres_least_squares.restype = None
     lib.bis_host_gmres_update_g.argtypes = [C.c_int, C.c_int] + [C.c_void_p] * 3 + [C.c_double]
     lib.bis_host_gmres_update_g.restype = C.c_double
+    lib.bis_host_gmres_back_substitution.argtypes = [C.c_int, C.c_int] + [C.c_void_p] * 3
+    lib.bis_host_gmres_back_substitution.restype = None
     lib.bis_host_solve.argtypes = ([C.c_void_p, C.c_char_p, C.c_int] + [C.c_void_p] * 3 + [C.c_int] * 3 +
                                    [C.c_void_p] * 2 + [C.c_int, C.c_double, C.c_int, C.c_int] + [C.c_void_p] * 5)
     lib.bis_host_solve_block.argtypes = ([C.c_void_p, C.c_char_p, C.c_int] + [C.c_void_p] * 3 + [C.c_int] * 2 +
                                          [C.c_void_p] * 2 + [C.c_int, C.c_double, C.c_int] + [C.c_void_p] * 7)
+    lib.bis_host_solve_block_gmres.argtypes = ([C.c_void_p, C.c_char_p, C.c_int] + [C.c_void_p] * 3 + [C.c_int] * 3 +
+                                               [C.c_void_p] * 2 + [C.c_int, C.c_double, C.c_int] + [C.c_void_p] * 8)
     lib.bis_host_bench_open.argtypes = [C.c_void_p, C.c_char_p, C.c_int, C.c_int, C.c_int]
     lib.bis_host_bench_open.restype = C.c_void_p
     lib.bis_host_bench_close.argtypes = [C.c_void_p]
@@ -143,6 +147,11 @@ def gmres_update_g(k, m, Q, g, g_tmp, beta) -> float:
     return load().bis_host_gmres_update_g(k, m, _p(Q), _p(g), _p(g_tmp), float(beta))
 
 
+def gmres_back_substitution(k, m, R, g, y):
+    """y[0:k] from R y = g (get_explicit_x of host/methods/gmres.hpp), R (m+1) x m row-major."""
+    load().bis_host_gmres_back_substitution(k, m, _p(R), _p(g), _p(y))
+
+
 @dataclass
 class SolveResult:
     history: np.ndarray          # collected_residual_norms[0:count]
@@ -201,7 +210,7 @@ def solve(ctx: capi.Context, method: str, precond: str = "none", *, crs=None, ma
 
 @dataclass
 class BlockSolveResult:
-    histories: list              # per column: residual norms ||r_0|| .. ||r_{iter_count}||
+    histories: list              # per column: residual norms ||r_0|| .. ||r_{iter_count}|| (GMRES: and each restart's)
     iter_counts: np.ndarray      # per column
     converged: np.ndarray        # per column (bool)
     final_true_residuals: np.ndarray   # per column ||b_j - A x*_j||
@@ -209,9 +218,12 @@ class BlockSolveResult:
     solve_time: float            # seconds: initial residual, iterations, read-backs
     launches: int
     iterations: int              # passes of the loop (the largest iter_count)
+    restarts: np.ndarray | None = None   # per column (GMRES)
 
 
-def _solve_block(ctx, precond, crs, matrix_name, B, X0, max_iters, tol, want_x, timer_from):
+def _solve_block(ctx, precond, crs, matrix_name, B, X0, max_iters, tol, want_x, timer_from, method, restart_len):
+    if method not in ("cg", "gm"):
+        raise ValueError(f"solve_block: method {method!r} not supported (cg or gm)")
     lib = load()
     B = np.ascontiguousarray(B, np.float64)
     if B.ndim == 1:
@@ -239,28 +251,47 @@ def _solve_block(ctx, precond, crs, matrix_name, B, X0, max_iters, tol, want_x, 
     xs = np.zeros((n, k)) if want_x else None
     od = np.zeros(4)
     oi = np.zeros(4, np.int64)
-    rc = lib.bis_host_solve_block(ctx.h, name, n, _p(rp), _p(col), _p(val), k, PRECOND[precond], _p(B), _p(X0),
-                                  int(max_iters), float(tol), int(timer_from), _p(hist), _p(its), _p(conv), _p(fres),
-                                  _p(xs), _p(od), _p(oi))
+    if method == "gm":
+        rst = np.zeros(k, np.int32)
+        rc = lib.bis_host_solve_block_gmres(ctx.h, name, n, _p(rp), _p(col), _p(val), k, PRECOND[precond],
+                                            int(restart_len), _p(B), _p(X0), int(max_iters), float(tol), int(timer_from),
+                                            _p(hist), _p(its), _p(conv), _p(rst), _p(fres), _p(xs), _p(od), _p(oi))
+    else:
+        rst = None
+        rc = lib.bis_host_solve_block(ctx.h, name, n, _p(rp), _p(col), _p(val), k, PRECOND[precond], _p(B), _p(X0),
+                                      int(max_iters), float(tol), int(timer_from), _p(hist), _p(its), _p(conv),
+                                      _p(fres), _p(xs), _p(od), _p(oi))
     if rc != 0:
         raise capi.BisError(_err())
-    res = BlockSolveResult([hist[j, :its[j] + 1].copy() for j in range(k)], its.astype(np.int64), conv.astype(bool),
-                           fres, xs, float(od[0]), int(oi[0]), int(oi[2]))
-    return res, float(od[1]), int(oi[3])
+    lens = its + 1 if rst is None else its + 1 + rst
+    res = BlockSolveResult([hist[j, :lens[j]].copy() for j in range(k)], its.astype(np.int64), conv.astype(bool),
+                           fres, xs, float(od[0]), int(oi[0]), int(oi[2]),
+                           None if rst is None else rst.astype(np.int64))
+    return res, float(od[1]), int(oi[3]), float(od[2])
 
 
 def solve_block(ctx: capi.Context, precond: str = "none", *, crs=None, matrix_name=None, B, X0=None,
-                max_iters: int = 0, tol: float = 0.0, want_x: bool = True) -> BlockSolveResult:
-    """CG on the k columns of B (an (n, k) array) with one matrix (host/methods/block_cg.hpp), precond "none"
-    or "j".  Every column runs the single-RHS CG's arithmetic and stop rule; the columns share one SpMM per
-    iteration.  X0: (n, k) or None (INIT_X_VAL).  max_iters <= 0 / tol <= 0 keep MAX_ITERS / TOL."""
-    return _solve_block(ctx, precond, crs, matrix_name, B, X0, max_iters, tol, want_x, 0)[0]
+                max_iters: int = 0, tol: float = 0.0, want_x: bool = True, method: str = "cg",
+                restart_len: int = 10) -> BlockSolveResult:
+    """A Krylov solve on the k columns of B (an (n, k) array) with one matrix, precond "none" or "j":
+    method "cg" (host/methods/block_cg.hpp) or "gm", GMRES restarted every `restart_len` (1..64) iterations
+    (host/methods/block_gmres.hpp).  Every column runs the single-RHS method's arithmetic, stop rule and restarts;
+    the columns share one SpMM per iteration.  X0: (n, k) or None (INIT_X_VAL).  max_iters <= 0 / tol <= 0 keep
+    MAX_ITERS / TOL."""
+    return _solve_block(ctx, precond, crs, matrix_name, B, X0, max_iters, tol, want_x, 0, method, restart_len)[0]
 
 
-def bench_block(ctx: capi.Context, matrix_name: str, B, precond: str = "none", warmup: int = 5, steps: int = 50):
-    """Measurement: exactly warmup + steps block-CG iterations (tolerance 0) on a named matrix; device time of
-    the last `steps` between CUDA events.  Returns (BlockSolveResult without x_star, timed ms, timed iterations)."""
-    return _solve_block(ctx, precond, None, matrix_name, B, None, warmup + steps, 0.0, False, warmup)
+def bench_block(ctx: capi.Context, matrix_name: str, B, precond: str = "none", warmup: int = 5, steps: int = 50,
+                method: str = "cg", restart_len: int = 10, stats: dict | None = None):
+    """Measurement: exactly warmup + steps block iterations (tolerance 0; GMRES: fewer by its restart count, as
+    the single-RHS stop rule has it) on a named matrix; device time of the iterations after the first `warmup`
+    between CUDA events.  Returns (BlockSolveResult without x_star, timed ms, timed iterations).  stats, if given,
+    receives "host_givens_s": host seconds of the GMRES Givens updates over the whole solve."""
+    res, ms, iters, givens_s = _solve_block(ctx, precond, None, matrix_name, B, None, warmup + steps, 0.0, False,
+                                            warmup, method, restart_len)
+    if stats is not None:
+        stats["host_givens_s"] = givens_s
+    return res, ms, iters
 
 
 def harness_trace(run_ahead: bool, max_iters: int, tol: float, decay: float):

@@ -3,6 +3,7 @@
 // tests and bench.py).  Device work goes through the C-ABI of libbis_b200.so.
 #include "lu_factors.hpp"
 #include "methods/block_cg.hpp"
+#include "methods/block_gmres.hpp"
 #include "run.hpp"
 
 #include <cstring>
@@ -156,6 +157,9 @@ double bis_host_gmres_update_g(int k, int m, double *Q, double *g, double *g_tmp
     update_g(k, m, Q, g, g_tmp, rn, beta);
     return rn;
 }
+void bis_host_gmres_back_substitution(int k, int m, const double *R, const double *g, double *y) {
+    back_substitution(k, m, R, g, y);
+}
 
 // A whole solve on the device.  Matrix: host CRS arrays (rp != NULL) or a
 // generator / file name.  b / x0: host vectors or NULL (B_VAL / INIT_X_VAL).
@@ -231,6 +235,27 @@ int bis_host_solve(bis_context *dev, const char *matrix_name, int n, const int *
     }
 }
 
+// The matrix of a multi-RHS solve on the device: host CRS arrays (rp != NULL) or a generator / file name; n > 0 must
+// be its row count.
+static std::unique_ptr<DeviceCRS> block_matrix(Args *args, bis_context *dev, int n, const int *rp, const int *col,
+                                               const double *val, const char *what) {
+    std::unique_ptr<MatrixCRS> A;
+    std::unique_ptr<DeviceCRS> dA;
+    if (rp) {
+        A = std::make_unique<MatrixCRS>(n, n, rp[n]);
+        std::memcpy(A->row_ptr, rp, sizeof(int) * (n + 1));
+        std::memcpy(A->col, col, sizeof(int) * rp[n]);
+        std::memcpy(A->val, val, sizeof(double) * rp[n]);
+        dA = upload_crs(dev, A.get());
+    } else {
+        obtain_matrix(args, dev, A, dA);
+        if (A) dA = upload_crs(dev, A.get());
+    }
+    if (n > 0 && dA->n_rows != n)
+        bis_fatal(std::string(what) + ": B has " + std::to_string(n) + " rows, the matrix " + std::to_string(dA->n_rows));
+    return dA;
+}
+
 // CG on k right-hand sides with one matrix (methods/block_cg.hpp).  Matrix: host CRS arrays (rp != NULL) or a
 // generator / file name, as bis_host_solve.  B: n x k row-major host array; X0 likewise or NULL (INIT_X_VAL).
 // precond: none or jacobi.  max_iters <= 0 keeps MAX_ITERS; tol <= 0 keeps TOL.
@@ -264,24 +289,7 @@ int bis_host_solve_block(bis_context *dev, const char *matrix_name, int n, const
             if (timer_from >= solver.max_iters) bis_fatal("block CG: timer_from must be below max_iters");
             solver.tolerance = 0.0;   // never stop early: exactly max_iters iterations
         }
-        std::unique_ptr<MatrixCRS> A;
-        std::unique_ptr<DeviceCRS> dA;
-        if (rp) {
-            A = std::make_unique<MatrixCRS>(n, n, rp[n]);
-            std::memcpy(A->row_ptr, rp, sizeof(int) * (n + 1));
-            std::memcpy(A->col, col, sizeof(int) * rp[n]);
-            std::memcpy(A->val, val, sizeof(double) * rp[n]);
-            dA = upload_crs(dev, A.get());
-            A.reset();
-        } else {
-            obtain_matrix(&args, dev, A, dA);
-            if (A) {
-                dA = upload_crs(dev, A.get());
-                A.reset();
-            }
-        }
-        if (n > 0 && dA->n_rows != n) bis_fatal("block CG: B has " + std::to_string(n) + " rows, the matrix " +
-                                               std::to_string(dA->n_rows));
+        std::unique_ptr<DeviceCRS> dA = block_matrix(&args, dev, n, rp, col, val, "block CG");
         int64_t info0[8], info1[8];
         BIS_OK(bis_context_info(dev, info0));
         Stopwatch w;
@@ -302,6 +310,72 @@ int bis_host_solve_block(bis_context *dev, const char *matrix_name, int n, const
             final_res[j] = fr[(size_t)j];
         }
         if (x_star) BIS_OK(bis_vector_download(dev, x_star, solver.X_old, solver.N * k));
+        out_int[0] = info1[3] - info0[3];
+        out_int[1] = solver.N;
+        out_int[2] = solver.iter_count;
+        out_int[3] = timed_iters;
+        return 0;
+    } catch (const std::exception &e) {
+        g_host_err = e.what();
+        return 1;
+    }
+}
+
+// Restarted GMRES on k right-hand sides with one matrix (methods/block_gmres.hpp).  Arguments and outputs as
+// bis_host_solve_block, plus restart_len (1..64) and restarts[j], the restarts of column j; column j's history holds
+// iter_count[j] + 1 + restarts[j] residual norms (r0, one per iteration, and the beta of every restart).
+// out_dbl: [0] solve seconds, [1] timed device ms, [2] host seconds in the Givens updates (least_squares and update_g,
+// all columns and iterations).  out_int as bis_host_solve_block.
+int bis_host_solve_block_gmres(bis_context *dev, const char *matrix_name, int n, const int *rp, const int *col,
+                               const double *val, int k, int precond, int restart_len, const double *B,
+                               const double *X0, int max_iters, double tol, int timer_from, double *history,
+                               int *iter_count, int *converged, int *restarts, double *final_res, double *x_star,
+                               double *out_dbl, int64_t *out_int) {
+    try {
+        Args args;
+        args.matrix_file_name = matrix_name ? matrix_name : "in-memory";
+        args.method = SolverType::GMRES;
+        args.preconditioner = static_cast<PrecondType>(precond);
+        args.restart_length = restart_len;
+        args.quiet = true;
+        if (!B) bis_fatal("block GMRES: B is required");
+        int perm_mode = 0;
+        BIS_OK(bis_context_get_option(dev, "perm_mode", &perm_mode));
+        if (perm_mode != 0) bis_fatal("block GMRES: perm_mode is not supported with several right-hand sides");
+        BlockGMRESSolver solver(&args, dev, k);
+        if (max_iters > 0) {
+            if (max_iters > MAX_ITERS) bis_fatal("max_iters exceeds MAX_ITERS");
+            solver.max_iters = max_iters;
+        }
+        if (tol > 0) solver.tolerance = tol;
+        if (timer_from > 0) {
+            if (timer_from >= solver.max_iters) bis_fatal("block GMRES: timer_from must be below max_iters");
+            solver.tolerance = 0.0;   // never stop on the norm
+        }
+        std::unique_ptr<DeviceCRS> dA = block_matrix(&args, dev, n, rp, col, val, "block GMRES");
+        int64_t info0[8], info1[8];
+        BIS_OK(bis_context_info(dev, info0));
+        Stopwatch w;
+        w.start();
+        solver.setup(std::move(dA), B, X0);
+        double timed_ms = 0.0;
+        int timed_iters = 0;
+        solver.run(timer_from, &timed_ms, &timed_iters);
+        out_dbl[0] = w.check();
+        out_dbl[1] = timed_ms;
+        out_dbl[2] = solver.givens_s;
+        BIS_OK(bis_context_info(dev, info1));
+        const std::vector<double> fr = solver.true_residuals();
+        for (int j = 0; j < k; ++j) {
+            const BlockGMRESSolver::Column &c = solver.col[(size_t)j];
+            for (size_t i = 0; i < c.history.size() && i < (size_t)(2 * MAX_ITERS); ++i)
+                history[(size_t)j * 2 * MAX_ITERS + i] = c.history[i];
+            iter_count[j] = c.iters;
+            converged[j] = c.converged ? 1 : 0;
+            restarts[j] = c.restarts;
+            final_res[j] = fr[(size_t)j];
+        }
+        if (x_star) BIS_OK(bis_vector_download(dev, x_star, solver.X, solver.N * k));
         out_int[0] = info1[3] - info0[3];
         out_int[1] = solver.N;
         out_int[2] = solver.iter_count;

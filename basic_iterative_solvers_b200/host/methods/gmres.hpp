@@ -46,6 +46,19 @@ inline void update_g(int n_solver_iters, int restart_len, double *Q, double *g, 
     residual_norm = std::abs(g[n_solver_iters + 1]);
 }
 
+// gmres.hpp:335-349: the k x k back-substitution R y = g of get_explicit_x
+inline void back_substitution(int k, int m, const double *R, const double *g, double *y) {
+    double diag_elem = 1.0;
+    for (int row = k - 1; row >= 0; --row) {
+        double sum = 0.0;
+        for (int c = row; c < k; ++c) {
+            if (row == c) diag_elem = R[row * m + c];
+            else sum = std::fma(R[row * m + c], y[c], sum);
+        }
+        y[row] = (g[row] - sum) / diag_elem;
+    }
+}
+
 class GMRESSolver : public Solver {
   public:
     double *x = nullptr, *x_old = nullptr, *V = nullptr, *Vy = nullptr, *w = nullptr;   // [dev]
@@ -164,15 +177,7 @@ class GMRESSolver : public Solver {
     void get_explicit_x() override {
         const int m = gmres_restart_len;
         const int k = iter_count - gmres_restart_count * m;
-        double diag_elem = 1.0;
-        for (int row = k - 1; row >= 0; --row) {
-            double sum = 0.0;
-            for (int c = row; c < k; ++c) {
-                if (row == c) diag_elem = R[row * m + c];
-                else sum = std::fma(R[row * m + c], y[c], sum);
-            }
-            y[row] = (g[row] - sum) / diag_elem;
-        }
+        back_substitution(k, m, R.data(), g.data(), y.data());
         BIS_OK(bis_gmres_update_x(dev, N, k, V, y.data(), x, x_old, Vy));
     }
 

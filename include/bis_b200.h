@@ -331,6 +331,14 @@ int bis_scalar_get(bis_context *ctx, int first_slot, int count,
 int bis_scalar_read_begin(bis_context *ctx, int first_slot, int count);
 int bis_scalar_read_end(bis_context *ctx, int first_slot, int count,
                         double *values /* [host] */);
+/* The same split read for `count` doubles of device memory at `src` (a block
+ * GMRES's Hessenberg column): one copy into a pinned staging buffer of the
+ * context plus an event.  count <= BIS_VECTOR_READ_MAX; _end must name the
+ * count of its _begin.  One vector read may be outstanding per context, next to
+ * one scalar read. */
+#define BIS_VECTOR_READ_MAX 4096
+int bis_vector_read_begin(bis_context *ctx, const double *src /* [dev] */, int64_t count);
+int bis_vector_read_end(bis_context *ctx, double *dst /* [host] */, int64_t count);
 int bis_scalar_copy(bis_context *ctx, int dst_slot, int src_slot);
 /* slot <- sum a*b ; slot <- sum v*v (NOT the square root) */
 int bis_dot_to_slot(bis_context *ctx, const double *a, const double *b,
@@ -494,6 +502,42 @@ int bis_block_cg_direction_x(bis_context *ctx, int64_t n, int k, double *P_new,
  * column still active counts the iteration. */
 int bis_block_cg_status(bis_context *ctx, int k, int slot_rr0, int max_iters,
                         double *state /* [dev] */);
+
+/* Block GMRES (restart length m <= BIS_BLOCK_GMRES_MAX_M): column j runs the
+ * arithmetic of the single-RHS GMRES on b_j.
+ *
+ * Basis: m+1 blocks of n x k, block l at V + l*ldv; ldv >= n*k must be even so
+ * that every block is 16-byte aligned.  Hessenberg: a caller-owned device array
+ * H of (m+2)*k doubles, entry (l, j) at H[l*k + j]; the kernels read their
+ * coefficients from it and reduce into it (not the scalar slots).
+ * `active` [dev]: k flags (1.0 / 0.0) or NULL = every column active.  A column
+ * that is not active is frozen: none of its W, V or H entries is written. */
+#define BIS_BLOCK_GMRES_MAX_M 64
+/* W = M^-1 W (NONE: W untouched; JACOBI: W / (1.0*A_D), as
+ * bis_apply_preconditioner), then H[0,j] <- (W_j, V0_j), or (W_j, W_j) when
+ * V0 == NULL.  Precond NONE or JACOBI only. */
+int bis_block_gmres_precond_dot(bis_context *ctx, int precond, int64_t n, int k,
+                                double *W, const double *A_D, const double *V0,
+                                double *H, const double *active);
+/* bis_mgs_step per column, 0 <= l < BIS_BLOCK_GMRES_MAX_M: W -= H[l,j] V_l,
+ * then H[l+1,j] <- (W_j, V_next_j), or (W_j, W_j) when V_next == NULL. */
+int bis_block_mgs_step(bis_context *ctx, int64_t n, int k, double *W,
+                       const double *V_l, const double *V_next, double *H, int l,
+                       const double *active);
+/* bis_scale_inv_norm per column, 0 <= l <= BIS_BLOCK_GMRES_MAX_M:
+ * out_j = W_j * (1.0 / sqrt(H[l,j])). */
+int bis_block_scale_inv_norm(bis_context *ctx, int64_t n, int k, double *out,
+                             const double *W, const double *H, int l,
+                             const double *active);
+/* bis_gmres_update_x per column j with mask[j] != 0: X_j = X_old_j +
+ * sum_{l<nb} V_l,j Y[j*nb + l] (products rounded, added left to right);
+ * other columns untouched.  nb <= BIS_BLOCK_GMRES_MAX_M; Y [host] k x nb and
+ * mask [host] k are copied into the launch (not retained, so this call is not
+ * for graph recording).  X may equal X_old. */
+int bis_block_gmres_update_x(bis_context *ctx, int64_t n, int k, int nb,
+                             const double *V, int64_t ldv,
+                             const double *Y /* [host] */, double *X,
+                             const double *X_old, const int *mask /* [host] */);
 
 #ifdef __cplusplus
 }
