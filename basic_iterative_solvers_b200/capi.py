@@ -123,6 +123,9 @@ _SIGS = {
     "bis_block_cg_update": ([c_ctx, cint, i64, cint] + [c_dev] * 5 + [cint] * 4 + [c_dev], cint),
     "bis_block_cg_direction_x": ([c_ctx, i64, cint] + [c_dev] * 5 + [cint] * 3 + [c_dev], cint),
     "bis_block_cg_status": ([c_ctx, cint, cint, cint, c_dev], cint),
+    "bis_spmm_sub": ([c_ctx, c_mat, cint, c_dev, c_dev, c_dev], cint),
+    "bis_block_sptrsv": ([c_ctx, c_mat, cint] + [c_dev] * 4, cint),
+    "bis_block_bsptrsv": ([c_ctx, c_mat, cint] + [c_dev] * 4, cint),
     "bis_block_gmres_precond_dot": ([c_ctx, cint, i64, cint] + [c_dev] * 5, cint),
     "bis_block_mgs_step": ([c_ctx, i64, cint] + [c_dev] * 4 + [cint, c_dev], cint),
     "bis_block_scale_inv_norm": ([c_ctx, i64, cint] + [c_dev] * 3 + [cint, c_dev], cint),

@@ -49,6 +49,7 @@ struct SpmmIn {
     const int *col;
     const double *val;
     const double *X;
+    const double *B;   // Y = B - A X per column (bis_spmm_sub), or nullptr: Y = A X
     double *Y;
     int64_t n_rows;
     int cap;
@@ -78,18 +79,27 @@ __device__ __forceinline__ void spmm_gather(const double *__restrict__ X, int c,
     }
 }
 
+// Y = acc, or Y = sub_rn(B, acc) (EpiSub of bis_spmv.cu) when B is given
 template <int K>
-__device__ __forceinline__ void spmm_store(double *__restrict__ Y, int64_t row, int c0, const double (&acc)[SpmmShape<K>::CW]) {
+__device__ __forceinline__ void spmm_store(double *__restrict__ Y, const double *B, int64_t row, int c0,
+                                           const double (&acc)[SpmmShape<K>::CW]) {
     using S = SpmmShape<K>;
     double *p = Y + row * K + c0;
     if constexpr (S::VEC) {
 #pragma unroll
         for (int w = 0; w < S::CW; w += 2)
-            if (c0 + w < K) *reinterpret_cast<double2 *>(p + w) = make_double2(acc[w], acc[w + 1]);
+            if (c0 + w < K) {
+                double2 v = make_double2(acc[w], acc[w + 1]);
+                if (B) {
+                    const double2 b = *reinterpret_cast<const double2 *>(B + row * K + c0 + w);
+                    v = make_double2(sub_rn(b.x, v.x), sub_rn(b.y, v.y));
+                }
+                *reinterpret_cast<double2 *>(p + w) = v;
+            }
     } else {
 #pragma unroll
         for (int w = 0; w < S::CW; ++w)
-            if (c0 + w < K) p[w] = acc[w];
+            if (c0 + w < K) p[w] = B ? sub_rn(B[row * K + c0 + w], acc[w]) : acc[w];
     }
 }
 
@@ -212,7 +222,7 @@ __global__ void __launch_bounds__(512, 1) spmm_tma_kernel(SpmmIn in) {
             double acc[S::CW];
             spmm_row<K>(in.X, ks - base, ke - base, c0, [&](int64_t k) { return sc[k]; },
                         [&](int64_t k) { return sv[k]; }, acc);
-            spmm_store<K>(in.Y, row, c0, acc);
+            spmm_store<K>(in.Y, in.B, row, c0, acc);
         }
         __syncthreads();   // every thread is done with stage `st`
         if (threadIdx.x == 0 && j + in.nstage < my_tiles) issue(j + in.nstage, is, ie);
@@ -234,7 +244,7 @@ __global__ void __launch_bounds__(256) spmm_direct_kernel(SpmmIn in) {
         double acc[S::CW];
         spmm_row<K>(in.X, (int64_t)rp[row], (int64_t)rp[row + 1], c0, [&](int64_t k) { return ld_stream(col + k); },
                     [&](int64_t k) { return ld_stream(val + k); }, acc);
-        spmm_store<K>(in.Y, row, c0, acc);
+        spmm_store<K>(in.Y, in.B, row, c0, acc);
     }
 }
 
@@ -255,10 +265,10 @@ bool spmm_plan(const bis_matrix *A, int tpr, int *rows, int *cap, size_t *smem) 
 }
 
 template <typename RP, int K>
-int launch_spmm(bis_context *c, const bis_matrix *A, const double *X, double *Y) {
+int launch_spmm(bis_context *c, const bis_matrix *A, const double *X, const double *B, double *Y) {
     using S = SpmmShape<K>;
     SpmmIn in;
-    in.rp = A->d_rp; in.col = A->d_col; in.val = A->d_val; in.X = X; in.Y = Y; in.n_rows = A->n_rows;
+    in.rp = A->d_rp; in.col = A->d_col; in.val = A->d_val; in.X = X; in.B = B; in.Y = Y; in.n_rows = A->n_rows;
     in.cap = 0; in.nstage = 2; in.rows = 0;
     int R = 0, cap = 0;
     size_t smem = 0;
@@ -621,9 +631,9 @@ int launch_block(bis_context *c, int k, const BlockArgs &a) {
 }
 
 template <typename RP>
-int launch_spmm_rp(bis_context *c, const bis_matrix *A, int k, const double *X, double *Y) {
+int launch_spmm_rp(bis_context *c, const bis_matrix *A, int k, const double *X, const double *B, double *Y) {
     switch (k) {
-#define BIS_SPMM_CASE(K) case K: return launch_spmm<RP, K>(c, A, X, Y);
+#define BIS_SPMM_CASE(K) case K: return launch_spmm<RP, K>(c, A, X, B, Y);
     BIS_SPMM_CASE(1) BIS_SPMM_CASE(2) BIS_SPMM_CASE(3) BIS_SPMM_CASE(4) BIS_SPMM_CASE(5) BIS_SPMM_CASE(6)
     BIS_SPMM_CASE(7) BIS_SPMM_CASE(8) BIS_SPMM_CASE(9) BIS_SPMM_CASE(10) BIS_SPMM_CASE(11) BIS_SPMM_CASE(12)
     BIS_SPMM_CASE(13) BIS_SPMM_CASE(14) BIS_SPMM_CASE(15) BIS_SPMM_CASE(16)
@@ -658,21 +668,31 @@ BlockArgs block_args(bis_context *c, int64_t n) {
 #define REQ_SLOTS(s, k, what) \
     BIS_REQUIRE((s) >= 0 && (s) + (k) <= BIS_NUM_SCALARS, "multi-RHS: slots %s [%d, %d) outside [0, %d)", what, (s), (s) + (k), BIS_NUM_SCALARS)
 
-extern "C" int bis_spmm(bis_context *c, const bis_matrix *A, int k, const double *X, double *Y) {
+static int spmm_entry(bis_context *c, const bis_matrix *A, int k, const double *X, const double *B, double *Y,
+                      const char *what) {
     REQ_BLOCK(c, k);
-    BIS_REQUIRE(A, "bis_spmm: null matrix");
-    BIS_REQUIRE(!A->distributed, "bis_spmm: distributed matrices are not supported");
+    BIS_REQUIRE(A, "%s: null matrix", what);
+    BIS_REQUIRE(!A->distributed, "%s: distributed matrices are not supported", what);
     BIS_REQUIRE_CRS(A);
     REQ_BLOCK_VEC(X, "X");
     REQ_BLOCK_VEC(Y, "Y");
-    BIS_REQUIRE(X != Y, "bis_spmm: X and Y must not alias");
-    BisNvtxRange nvtx_range("spmm");
+    BIS_REQUIRE(X != Y, "%s: X and Y must not alias", what);
+    BisNvtxRange nvtx_range(what + 4);
     BIS_CUDA(cudaSetDevice(c->device));
     BIS_CHECK(bis_prof_begin(c, BIS_PROF_SPMV));
-    if (A->rp_bytes == 8) BIS_CHECK(launch_spmm_rp<int64_t>(c, A, k, X, Y));
-    else BIS_CHECK(launch_spmm_rp<int32_t>(c, A, k, X, Y));
+    if (A->rp_bytes == 8) BIS_CHECK(launch_spmm_rp<int64_t>(c, A, k, X, B, Y));
+    else BIS_CHECK(launch_spmm_rp<int32_t>(c, A, k, X, B, Y));
     BIS_CHECK(bis_prof_end(c, BIS_PROF_SPMV));
     return 0;
+}
+
+extern "C" int bis_spmm(bis_context *c, const bis_matrix *A, int k, const double *X, double *Y) {
+    return spmm_entry(c, A, k, X, nullptr, Y, "bis_spmm");
+}
+
+extern "C" int bis_spmm_sub(bis_context *c, const bis_matrix *T, int k, const double *X, const double *B, double *Y) {
+    REQ_BLOCK_VEC(B, "B");
+    return spmm_entry(c, T, k, X, B, Y, "bis_spmm_sub");
 }
 
 extern "C" int bis_block_dot_to_slots(bis_context *c, int64_t n, int k, const double *A, const double *B, int slot0,

@@ -271,6 +271,12 @@ struct LevelSets {
     double *d_w2 = nullptr;           // its twin: solves alternate between the two, each resets the other one while it runs
     int w_clean[2] = {1, 1};          // host's knowledge: that working vector holds "not ready" everywhere
     uint64_t w_epoch = 0;             // ... valid while the context's graph_epoch has this value
+    // working arrays of the multi-RHS solve (bis_block_sptrsv): n_slots x bw_k doubles each, slot-major, allocated on
+    // first use for the largest k seen; bw_dirty[i]: elements [0, bw_dirty[i]) may hold values (0: all "not ready")
+    double *d_bw[2] = {nullptr, nullptr};
+    int bw_k = 0;
+    int64_t bw_dirty[2] = {0, 0};
+    uint64_t bw_epoch = 0;
     // level-ordered copy of the strict factor (rows stored in slot order, operands named by slot)
     int64_t *d_rp = nullptr;          // [n_slots+1]
     int *d_col = nullptr;

@@ -39,6 +39,8 @@ void free_matrix_storage(bis_matrix *A) {
     cudaFree(A->lv.d_ticket);
     cudaFree(A->lv.d_w);
     cudaFree(A->lv.d_w2);
+    cudaFree(A->lv.d_bw[0]);
+    cudaFree(A->lv.d_bw[1]);
     cudaFree(A->lv.wave.d_rec);
     cudaFree(A->lv.wave.d_w[0]);
     cudaFree(A->lv.wave.d_w[1]);

@@ -707,6 +707,14 @@ int bis_wave_build(bis_context *c, const bis_matrix *T) {
     return wave_build_t<int32_t>(c, T);
 }
 
+// sleeps of the dataflow solves: per gate level distance, and between two polls of the missing operands
+static void trsv_wait_params(const bis_context *c, unsigned int gate_sleep[16], unsigned int *poll_ns) {
+    const int *sl = c->opt_trsv_sleep;
+    for (int d = 0; d < 16; ++d)
+        gate_sleep[d] = (unsigned int)(d <= 1 ? sl[0] : d == 2 ? sl[1] : d == 3 ? sl[2] : d < 6 ? sl[3] : 2 * sl[3]);
+    *poll_ns = c->opt_trsv_poll_ns > 0 ? (unsigned int)c->opt_trsv_poll_ns : (c->opt_trsv_poll_ns < 0 ? 0u : 20u);   // < 0: spin without sleeping
+}
+
 static int trsv_solve(bis_context *c, const bis_matrix *T, double *x, const double *D,
                       const double *b, int want_kind, int post_mul_d = 0) {
     BIS_REQUIRE(c && T && x && D && b, "sptrsv: null argument");
@@ -735,10 +743,7 @@ static int trsv_solve(bis_context *c, const bis_matrix *T, double *x, const doub
     a.slot_row = lv.d_slot_row;
     a.slot_level = lv.d_slot_level;
     a.gate = c->opt_trsv_gates ? reinterpret_cast<const int4 *>(lv.d_slot_gate) : nullptr;
-    for (int d = 0; d < 16; ++d) {
-        const int *sl = c->opt_trsv_sleep;
-        a.gate_sleep[d] = (unsigned int)(d <= 1 ? sl[0] : d == 2 ? sl[1] : d == 3 ? sl[2] : d < 6 ? sl[3] : 2 * sl[3]);
-    }
+    trsv_wait_params(c, a.gate_sleep, &a.poll_ns);
     a.rp = lv.d_rp;
     a.col = lv.d_col;
     a.val = lv.d_val;
@@ -747,7 +752,6 @@ static int trsv_solve(bis_context *c, const bis_matrix *T, double *x, const doub
     a.ticket = lv.d_ticket;
     a.errflag = c->d_errflag;
     a.dbg = nullptr;
-    a.poll_ns = c->opt_trsv_poll_ns > 0 ? (unsigned int)c->opt_trsv_poll_ns : (c->opt_trsv_poll_ns < 0 ? 0u : 20u);   // < 0: spin without sleeping
     const char *dbg_file = c->opt_trsv_debug ? getenv("BIS_TRSV_DEBUG_FILE") : nullptr;
     if (dbg_file) BIS_CUDA(bis_cuda_malloc(&a.dbg, sizeof(unsigned long long) * 4 * (size_t)lv.n_slots));
     a.x = x;
@@ -831,6 +835,303 @@ extern "C" int bis_sptrsv(bis_context *c, const bis_matrix *L, double *x, const 
 extern "C" int bis_bsptrsv(bis_context *c, const bis_matrix *U, double *x, const double *D,
                            const double *b) {
     return trsv_solve(c, U, x, D, b, 2);
+}
+
+// ---- several right-hand sides (bis_block_sptrsv / bis_block_bsptrsv) -----------------------------------
+// The dataflow solve above with k columns carried through every dependency: the same level-ordered copy, the same
+// ticket hand-out in slot order, the same "the value is its own ready flag" protocol, on a working array of
+// n_slots x k doubles (element (slot, j) at slot*k + j).  A row is served by TPR threads (1, 2, 4, 8 for k <= 2, 4, 8,
+// 16); each owns CW <= 2 consecutive columns and polls and publishes only those of them that are active.  The operands
+// of a window of PF = 16 nonzeros are polled together, warp-uniformly, and added in storage order; a row longer than
+// the window takes further windows, so the sum is that of the single-vector kernel for every column.  Two columns per
+// thread keep a whole HPCG factor row (13 nonzeros) in one window: with four columns per thread and an 8-nonzero
+// window (what the registers allow) the solve took 6.5 us per level at k = 4..16 against 1.7 us at k = 2 (HPCG-128).
+namespace {
+
+template <int K> struct BtrsvShape {
+    static constexpr int TPR = K <= 2 ? 1 : (K <= 4 ? 2 : (K <= 8 ? 4 : 8));   // threads per row
+    static constexpr int CW = (K + TPR - 1) / TPR;                              // columns per thread (<= 2)
+    static constexpr int PF = 16;                                               // nonzeros per window: PF * CW <= 32 poll bits
+    static constexpr int ROWS = 256 / TPR;                      // rows per block
+};
+
+struct BtrsvArgs {
+    int64_t n_slots;
+    const int *slot_row;
+    const int *slot_level;
+    const int4 *gate;
+    unsigned int gate_sleep[16];
+    unsigned int poll_ns;
+    const int64_t *rp;
+    const int *col;
+    const double *val;
+    unsigned int *ticket;
+    int *errflag;
+    double *X;
+    const double *D;
+    const double *B;
+    const double *active;   // [k] flags or nullptr
+    double *w_clean;        // the other working array: reset to "not ready" in [0, n_slots*k)
+};
+
+template <int K>
+__global__ void __launch_bounds__(256, 1) block_sptrsv_kernel(BtrsvArgs a, double *wk) {
+    using S = BtrsvShape<K>;
+    constexpr int CW = S::CW, PF = S::PF;
+    __shared__ unsigned int s_chunk;
+    if (threadIdx.x == 0) s_chunk = atomicAdd(a.ticket, 1u);
+    __syncthreads();
+    const int64_t slot = (int64_t)s_chunk * S::ROWS + threadIdx.x / S::TPR;
+    const int c0 = ((int)threadIdx.x % S::TPR) * CW;
+    const bool live = slot < a.n_slots;
+
+    unsigned int act = 0u;   // bit w: column c0 + w exists and is active
+#pragma unroll
+    for (int w = 0; w < CW; ++w)
+        if (c0 + w < K && (a.active == nullptr || a.active[c0 + w] != 0.0)) act |= 1u << w;
+    int row = 0, lvl = 0x7fffffff;
+    int64_t s = 0, e = 0;
+    double bb[CW], dd = 1.0;
+#pragma unroll
+    for (int w = 0; w < CW; ++w) bb[w] = 0.0;
+    if (live) {
+        row = a.slot_row[slot];
+        lvl = a.slot_level[slot];
+        s = a.rp[slot];
+        e = a.rp[slot + 1];
+        dd = a.D[row];
+#pragma unroll
+        for (int w = 0; w < CW; ++w) {
+            if (act >> w & 1u) bb[w] = a.B[(int64_t)row * K + c0 + w];
+            if (c0 + w < K) reinterpret_cast<unsigned long long *>(a.w_clean)[slot * K + c0 + w] = TRSV_SENTINEL;
+        }
+    } else {
+        act = 0u;
+    }
+    // the head of the row is in registers before anything is waited for
+    double av[PF];
+    int cv[PF];
+#pragma unroll
+    for (int j = 0; j < PF; ++j) {
+        const bool ok = act && s + j < e;
+        av[j] = ok ? __ldcs(a.val + s + j) : 0.0;
+        cv[j] = ok ? __ldcs(a.col + s + j) : -1;
+    }
+    int lv_lo = lvl, lv_hi = live ? lvl : -1;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        lv_lo = min(lv_lo, __shfl_xor_sync(0xffffffffu, lv_lo, o));
+        lv_hi = max(lv_hi, __shfl_xor_sync(0xffffffffu, lv_hi, o));
+    }
+    // staged waiting on the gates, through the first active column this thread owns
+    if (a.gate && act) {
+        const int wg = __ffs(act) - 1;
+        const int4 g = a.gate[slot];
+#pragma unroll
+        for (int i = 0; i < 3; ++i) {
+            const int gc = i == 0 ? g.x : (i == 1 ? g.y : g.z);
+            if (gc < 0) continue;
+            const unsigned int ns = a.gate_sleep[(g.w >> (8 * i)) & 15];
+            unsigned int spins = 0;
+            unsigned long long t_gate = 0;
+            while (ld_relaxed_u64(wk + (int64_t)gc * K + c0 + wg) == TRSV_SENTINEL) {
+                if (ns) __nanosleep(ns);
+                if ((++spins & 1023u) == 0) {
+                    if (t_gate == 0) t_gate = bis_globaltimer();
+                    if (*reinterpret_cast<volatile int *>(a.errflag)) break;
+                    if (bis_globaltimer() - t_gate > TRSV_WATCHDOG_NS) {
+                        atomicExch(a.errflag, 2);
+                        break;
+                    }
+                }
+            }
+        }
+    }
+    __syncwarp();
+    // operands: everything already published is taken now; operand (j, w) is bit j*CW + w of the poll mask
+    unsigned long long xv[PF][CW];
+    unsigned int miss = 0u;
+    auto take_window = [&]() {
+        miss = 0u;
+#pragma unroll
+        for (int j = 0; j < PF; ++j)
+#pragma unroll
+            for (int w = 0; w < CW; ++w) {
+                const bool use = cv[j] >= 0 && (act >> w & 1u);
+                xv[j][w] = use ? ld_relaxed_u64(wk + (int64_t)cv[j] * K + c0 + w) : 0ull;
+                if (use && xv[j][w] == TRSV_SENTINEL) miss |= 1u << (j * CW + w);
+            }
+    };
+    take_window();
+
+    for (int lv = lv_lo; lv <= lv_hi; ++lv) {
+        const bool mine = act && lvl == lv;
+        const int nwin = mine ? (int)((e - s + PF - 1) / PF) : 0;
+        const int nwin_max = __reduce_max_sync(0xffffffffu, (unsigned)nwin);
+        double sum[CW];
+#pragma unroll
+        for (int w = 0; w < CW; ++w) sum[w] = 0.0;
+        bool ok = true;
+        for (int win = 0; win < nwin_max && ok; ++win) {
+            if (win > 0 && mine && win < nwin) {   // the next window of a long row
+                const int64_t b0 = s + (int64_t)win * PF;
+#pragma unroll
+                for (int j = 0; j < PF; ++j) {
+                    const bool in = b0 + j < e;
+                    av[j] = in ? a.val[b0 + j] : 0.0;
+                    cv[j] = in ? a.col[b0 + j] : -1;
+                }
+                take_window();
+            }
+            const bool here = mine && win < nwin;
+            unsigned long long t_wd = 0;
+            unsigned int spins = 0;
+            // warp-uniform wait: the warp moves on when every row of this level has the operands of this window
+            for (;;) {
+                if (here && miss) {
+                    const unsigned int before = miss;
+#pragma unroll
+                    for (int j = 0; j < PF; ++j)
+#pragma unroll
+                        for (int w = 0; w < CW; ++w)
+                            if (miss & (1u << (j * CW + w))) xv[j][w] = ld_relaxed_u64(wk + (int64_t)cv[j] * K + c0 + w);
+#pragma unroll
+                    for (int j = 0; j < PF; ++j)
+#pragma unroll
+                        for (int w = 0; w < CW; ++w)
+                            if (xv[j][w] != TRSV_SENTINEL) miss &= ~(1u << (j * CW + w));
+                    if (miss != before) t_wd = 0;   // progress
+                }
+                if (__all_sync(0xffffffffu, !here || miss == 0u)) break;
+                if (a.poll_ns) __nanosleep(a.poll_ns);
+                bool give_up = false;
+                if ((++spins & 4095u) == 0) {
+                    if (t_wd == 0) t_wd = bis_globaltimer();
+                    give_up = *reinterpret_cast<volatile int *>(a.errflag) != 0 || bis_globaltimer() - t_wd > TRSV_WATCHDOG_NS;
+                }
+                if (__any_sync(0xffffffffu, give_up)) {
+                    atomicExch(a.errflag, 1);
+                    ok = false;
+                    break;
+                }
+            }
+            if (here && ok) {
+#pragma unroll
+                for (int j = 0; j < PF; ++j)
+                    if (cv[j] >= 0)
+#pragma unroll
+                        for (int w = 0; w < CW; ++w)
+                            sum[w] = add_rn(sum[w], mul_rn(av[j], __longlong_as_double((long long)xv[j][w])));
+            }
+        }
+        // a warp that gave up publishes nothing: its rows stay "not ready" and their readers give up too
+        if (mine && ok) {
+#pragma unroll
+            for (int w = 0; w < CW; ++w) {
+                if (!(act >> w & 1u)) continue;
+                const double r = div_rn(sub_rn(bb[w], sum[w]), dd);
+                __stcg(wk + slot * K + c0 + w, r);
+                a.X[(int64_t)row * K + c0 + w] = r;
+            }
+        }
+        __syncwarp();
+    }
+}
+
+template <int K>
+int launch_block_trsv(bis_context *c, const BtrsvArgs &a, double *wk) {
+    constexpr int R = BtrsvShape<K>::ROWS;
+    block_sptrsv_kernel<K><<<(unsigned int)((a.n_slots + R - 1) / R), 256, 0, c->stream>>>(a, wk);
+    BIS_LAUNCH_CHECK(c);
+    return 0;
+}
+
+} // namespace
+
+static int block_trsv_solve(bis_context *c, const bis_matrix *T, int k, double *X, const double *D, const double *B,
+                            const double *active, int want_kind) {
+    const char *what = want_kind == 1 ? "bis_block_sptrsv" : "bis_block_bsptrsv";
+    BIS_REQUIRE(c != nullptr, "null context");
+    BIS_REQUIRE(c->nranks == 1, "multi-RHS entry points are single-GPU only (distributed context)");
+    BIS_REQUIRE(k >= 1 && k <= BIS_BLOCK_MAX_K, "multi-RHS: k = %d outside [1, %d]", k, BIS_BLOCK_MAX_K);
+    BIS_REQUIRE(T && D, "%s: null argument", what);
+    BIS_REQUIRE(X && (reinterpret_cast<uintptr_t>(X) & 15) == 0, "multi-RHS: X is null or not 16-byte aligned");
+    BIS_REQUIRE(B && (reinterpret_cast<uintptr_t>(B) & 15) == 0, "multi-RHS: B is null or not 16-byte aligned");
+    BIS_REQUIRE(T->triangular == want_kind, "%s: matrix is not the %s strictly-triangular factor this call needs", what,
+                want_kind == 1 ? "lower" : "upper");
+    BIS_REQUIRE(!T->distributed, "%s: triangular sweeps do not shard (single-GPU only)", what);
+    BisNvtxRange nvtx_range(want_kind == 1 ? "block-sptrsv" : "block-backwards-sptrsv");
+    BIS_CUDA(cudaSetDevice(c->device));
+    if (T->n_rows == 0) return 0;
+    BIS_CHECK(bis_ensure_levels(c, T));
+    LevelSets &lv = T->lv;
+    const int64_t need = lv.n_slots * k;
+    if (lv.bw_k < k) {   // (re)allocated for the largest k so far; both arrays count as dirty until filled or reset
+        BIS_REQUIRE(!c->capturing, "%s: the first solve with %d columns must not be recorded into a graph", what, k);
+        BIS_CUDA(cudaStreamSynchronize(c->stream));
+        cudaFree(lv.d_bw[0]);
+        cudaFree(lv.d_bw[1]);
+        lv.d_bw[0] = lv.d_bw[1] = nullptr;
+        lv.bw_k = 0;
+        BIS_CUDA(bis_cuda_malloc(&lv.d_bw[0], sizeof(double) * (size_t)need));
+        BIS_CUDA(bis_cuda_malloc(&lv.d_bw[1], sizeof(double) * (size_t)need));
+        lv.bw_k = k;
+        lv.bw_dirty[0] = lv.bw_dirty[1] = need;
+        lv.bw_epoch = c->graph_epoch;
+    }
+    const int64_t full = lv.n_slots * lv.bw_k;
+    if (lv.bw_epoch != c->graph_epoch || c->capturing) {   // a graph replay may have used either array since
+        lv.bw_dirty[0] = lv.bw_dirty[1] = full;
+        lv.bw_epoch = c->graph_epoch;
+    }
+    BtrsvArgs a;
+    a.n_slots = lv.n_slots;
+    a.slot_row = lv.d_slot_row;
+    a.slot_level = lv.d_slot_level;
+    a.gate = c->opt_trsv_gates ? reinterpret_cast<const int4 *>(lv.d_slot_gate) : nullptr;
+    trsv_wait_params(c, a.gate_sleep, &a.poll_ns);
+    a.rp = lv.d_rp;
+    a.col = lv.d_col;
+    a.val = lv.d_val;
+    a.ticket = lv.d_ticket;
+    a.errflag = c->d_errflag;
+    a.X = X;
+    a.D = D;
+    a.B = B;
+    a.active = active;
+    BIS_CHECK(bis_prof_begin(c, BIS_PROF_SPTRSV));
+    int p = lv.bw_dirty[0] == 0 ? 0 : (lv.bw_dirty[1] == 0 ? 1 : -1);
+    if (p < 0) {   // neither is known to be clean: inside a graph, after one, or on first use
+        const int64_t cnt = std::max(lv.bw_dirty[0], need);
+        trsv_fill_sentinel_kernel<<<bis_blocks_for(cnt, 1024, c->sm_count * 8), 256, 0, c->stream>>>(cnt, lv.d_bw[0]);
+        BIS_LAUNCH_CHECK(c);
+        lv.bw_dirty[0] = 0;
+        p = 0;
+    }
+    a.w_clean = lv.d_bw[1 - p];
+    // this solve leaves values in [0, need) of its array and resets [0, need) of the other one
+    lv.bw_dirty[p] = need;
+    lv.bw_dirty[1 - p] = c->capturing ? full : (lv.bw_dirty[1 - p] <= need ? 0 : lv.bw_dirty[1 - p]);
+    BIS_CUDA(cudaMemsetAsync(lv.d_ticket, 0, sizeof(unsigned int), c->stream));
+    int rc = 2;
+    switch (k) {
+#define BIS_BTRSV_CASE(KK) case KK: rc = launch_block_trsv<KK>(c, a, lv.d_bw[p]); break;
+    BIS_BTRSV_CASE(1) BIS_BTRSV_CASE(2) BIS_BTRSV_CASE(3) BIS_BTRSV_CASE(4) BIS_BTRSV_CASE(5) BIS_BTRSV_CASE(6)
+    BIS_BTRSV_CASE(7) BIS_BTRSV_CASE(8) BIS_BTRSV_CASE(9) BIS_BTRSV_CASE(10) BIS_BTRSV_CASE(11) BIS_BTRSV_CASE(12)
+    BIS_BTRSV_CASE(13) BIS_BTRSV_CASE(14) BIS_BTRSV_CASE(15) BIS_BTRSV_CASE(16)
+#undef BIS_BTRSV_CASE
+    }
+    BIS_CHECK(rc);
+    return bis_prof_end(c, BIS_PROF_SPTRSV);
+}
+
+extern "C" int bis_block_sptrsv(bis_context *c, const bis_matrix *L, int k, double *X, const double *D, const double *B,
+                                const double *active) {
+    return block_trsv_solve(c, L, k, X, D, B, active, 1);
+}
+extern "C" int bis_block_bsptrsv(bis_context *c, const bis_matrix *U, int k, double *X, const double *D, const double *B,
+                                 const double *active) {
+    return block_trsv_solve(c, U, k, X, D, B, active, 2);
 }
 
 // two_stage_gauss_seidel, kernels.hpp:312-333: a truncated Neumann series for (D + T)^-1 -- SpMV only, no

@@ -50,6 +50,8 @@ def load() -> C.CDLL:
                                    [C.c_void_p] * 2 + [C.c_int, C.c_double, C.c_int, C.c_int] + [C.c_void_p] * 5)
     lib.bis_host_solve_block.argtypes = ([C.c_void_p, C.c_char_p, C.c_int] + [C.c_void_p] * 3 + [C.c_int] * 2 +
                                          [C.c_void_p] * 2 + [C.c_int, C.c_double, C.c_int] + [C.c_void_p] * 7)
+    lib.bis_host_solve_block_gs.argtypes = ([C.c_void_p, C.c_char_p, C.c_int] + [C.c_void_p] * 3 + [C.c_int] * 3 +
+                                            [C.c_void_p] * 2 + [C.c_int, C.c_double, C.c_int] + [C.c_void_p] * 7)
     lib.bis_host_solve_block_gmres.argtypes = ([C.c_void_p, C.c_char_p, C.c_int] + [C.c_void_p] * 3 + [C.c_int] * 3 +
                                                [C.c_void_p] * 2 + [C.c_int, C.c_double, C.c_int] + [C.c_void_p] * 8)
     lib.bis_host_bench_open.argtypes = [C.c_void_p, C.c_char_p, C.c_int, C.c_int, C.c_int]
@@ -222,8 +224,8 @@ class BlockSolveResult:
 
 
 def _solve_block(ctx, precond, crs, matrix_name, B, X0, max_iters, tol, want_x, timer_from, method, restart_len):
-    if method not in ("cg", "gm"):
-        raise ValueError(f"solve_block: method {method!r} not supported (cg or gm)")
+    if method not in ("cg", "gm", "gs", "sgs"):
+        raise ValueError(f"solve_block: method {method!r} not supported (cg, gm, gs or sgs)")
     lib = load()
     B = np.ascontiguousarray(B, np.float64)
     if B.ndim == 1:
@@ -256,6 +258,11 @@ def _solve_block(ctx, precond, crs, matrix_name, B, X0, max_iters, tol, want_x, 
         rc = lib.bis_host_solve_block_gmres(ctx.h, name, n, _p(rp), _p(col), _p(val), k, PRECOND[precond],
                                             int(restart_len), _p(B), _p(X0), int(max_iters), float(tol), int(timer_from),
                                             _p(hist), _p(its), _p(conv), _p(rst), _p(fres), _p(xs), _p(od), _p(oi))
+    elif method in ("gs", "sgs"):
+        rst = None
+        rc = lib.bis_host_solve_block_gs(ctx.h, name, n, _p(rp), _p(col), _p(val), k, PRECOND[precond],
+                                         int(method == "sgs"), _p(B), _p(X0), int(max_iters), float(tol), int(timer_from),
+                                         _p(hist), _p(its), _p(conv), _p(fres), _p(xs), _p(od), _p(oi))
     else:
         rst = None
         rc = lib.bis_host_solve_block(ctx.h, name, n, _p(rp), _p(col), _p(val), k, PRECOND[precond], _p(B), _p(X0),
@@ -273,18 +280,19 @@ def _solve_block(ctx, precond, crs, matrix_name, B, X0, max_iters, tol, want_x, 
 def solve_block(ctx: capi.Context, precond: str = "none", *, crs=None, matrix_name=None, B, X0=None,
                 max_iters: int = 0, tol: float = 0.0, want_x: bool = True, method: str = "cg",
                 restart_len: int = 10) -> BlockSolveResult:
-    """A Krylov solve on the k columns of B (an (n, k) array) with one matrix, precond "none" or "j":
-    method "cg" (host/methods/block_cg.hpp) or "gm", GMRES restarted every `restart_len` (1..64) iterations
-    (host/methods/block_gmres.hpp).  Every column runs the single-RHS method's arithmetic, stop rule and restarts;
-    the columns share one SpMM per iteration.  X0: (n, k) or None (INIT_X_VAL).  max_iters <= 0 / tol <= 0 keep
-    MAX_ITERS / TOL."""
+    """A solve on the k columns of B (an (n, k) array) with one matrix: method "cg" (host/methods/block_cg.hpp) or
+    "gm", GMRES restarted every `restart_len` (1..64) iterations (host/methods/block_gmres.hpp), with precond "none"
+    or "j"; or method "gs" / "sgs", Gauss-Seidel / symmetric Gauss-Seidel (host/methods/block_gs.hpp), precond
+    "none" only.  Every column runs the single-RHS method's arithmetic, stop rule and restarts; the columns share one
+    pass over the matrix (CG, GMRES) or over each triangular factor (GS, SGS) per iteration.  X0: (n, k) or None
+    (INIT_X_VAL).  max_iters <= 0 / tol <= 0 keep MAX_ITERS / TOL."""
     return _solve_block(ctx, precond, crs, matrix_name, B, X0, max_iters, tol, want_x, 0, method, restart_len)[0]
 
 
 def bench_block(ctx: capi.Context, matrix_name: str, B, precond: str = "none", warmup: int = 5, steps: int = 50,
                 method: str = "cg", restart_len: int = 10, stats: dict | None = None):
-    """Measurement: exactly warmup + steps block iterations (tolerance 0; GMRES: fewer by its restart count, as
-    the single-RHS stop rule has it) on a named matrix; device time of the iterations after the first `warmup`
+    """Measurement: exactly warmup + steps block iterations of `method` ("cg", "gm", "gs" or "sgs"; tolerance 0;
+    GMRES: fewer by its restart count, as the single-RHS stop rule has it) on a named matrix; device time of the iterations after the first `warmup`
     between CUDA events.  Returns (BlockSolveResult without x_star, timed ms, timed iterations).  stats, if given,
     receives "host_givens_s": host seconds of the GMRES Givens updates over the whole solve."""
     res, ms, iters, givens_s = _solve_block(ctx, precond, None, matrix_name, B, None, warmup + steps, 0.0, False,

@@ -4,6 +4,7 @@
 #include "lu_factors.hpp"
 #include "methods/block_cg.hpp"
 #include "methods/block_gmres.hpp"
+#include "methods/block_gs.hpp"
 #include "run.hpp"
 
 #include <cstring>
@@ -256,6 +257,55 @@ static std::unique_ptr<DeviceCRS> block_matrix(Args *args, bis_context *dev, int
     return dA;
 }
 
+// The part of a block CG / GS solve after its solver is made: options, matrix, setup, the loop, the outputs.
+extern "C++" {
+template <class BlockS>
+static void solve_block_with(BlockS &solver, Args *args, bis_context *dev, const char *what, int n, const int *rp,
+                             const int *col, const double *val, int k, const double *B, const double *X0, int max_iters,
+                             double tol, int timer_from, double *history, int *iter_count, int *converged,
+                             double *final_res, double *out_dbl, int64_t *out_int) {
+    if (max_iters > 0) {
+        if (max_iters > MAX_ITERS) bis_fatal("max_iters exceeds MAX_ITERS");
+        solver.max_iters = max_iters;
+    }
+    if (tol > 0) solver.tolerance = tol;
+    if (timer_from > 0) {
+        if (timer_from >= solver.max_iters) bis_fatal(std::string(what) + ": timer_from must be below max_iters");
+        solver.tolerance = 0.0;   // never stop early: exactly max_iters iterations
+    }
+    std::unique_ptr<DeviceCRS> dA = block_matrix(args, dev, n, rp, col, val, what);
+    int64_t info0[8], info1[8];
+    BIS_OK(bis_context_info(dev, info0));
+    Stopwatch w;
+    w.start();
+    solver.setup(std::move(dA), B, X0);
+    double timed_ms = 0.0;
+    int timed_iters = 0;
+    solver.run(timer_from, &timed_ms, &timed_iters);
+    out_dbl[0] = w.check();
+    out_dbl[1] = timed_ms;
+    BIS_OK(bis_context_info(dev, info1));
+    const std::vector<double> fr = solver.true_residuals();
+    for (int j = 0; j < k; ++j) {
+        const std::vector<double> &h = solver.col_history[(size_t)j];
+        for (size_t i = 0; i < h.size() && i < (size_t)(2 * MAX_ITERS); ++i) history[(size_t)j * 2 * MAX_ITERS + i] = h[i];
+        iter_count[j] = solver.col_iters[(size_t)j];
+        converged[j] = solver.col_converged[(size_t)j];
+        final_res[j] = fr[(size_t)j];
+    }
+    out_int[0] = info1[3] - info0[3];
+    out_int[1] = solver.N;
+    out_int[2] = solver.iter_count;
+    out_int[3] = timed_iters;
+}
+} // extern "C++"
+
+static void reject_perm_mode(bis_context *dev, const char *what) {
+    int perm_mode = 0;
+    BIS_OK(bis_context_get_option(dev, "perm_mode", &perm_mode));
+    if (perm_mode != 0) bis_fatal(std::string(what) + ": perm_mode is not supported with several right-hand sides");
+}
+
 // CG on k right-hand sides with one matrix (methods/block_cg.hpp).  Matrix: host CRS arrays (rp != NULL) or a
 // generator / file name, as bis_host_solve.  B: n x k row-major host array; X0 likewise or NULL (INIT_X_VAL).
 // precond: none or jacobi.  max_iters <= 0 keeps MAX_ITERS; tol <= 0 keeps TOL.
@@ -276,44 +326,37 @@ int bis_host_solve_block(bis_context *dev, const char *matrix_name, int n, const
         args.preconditioner = static_cast<PrecondType>(precond);
         args.quiet = true;
         if (!B) bis_fatal("block CG: B is required");
-        int perm_mode = 0;
-        BIS_OK(bis_context_get_option(dev, "perm_mode", &perm_mode));
-        if (perm_mode != 0) bis_fatal("block CG: perm_mode is not supported with several right-hand sides");
+        reject_perm_mode(dev, "block CG");
         BlockCGSolver solver(&args, dev, k);
-        if (max_iters > 0) {
-            if (max_iters > MAX_ITERS) bis_fatal("max_iters exceeds MAX_ITERS");
-            solver.max_iters = max_iters;
-        }
-        if (tol > 0) solver.tolerance = tol;
-        if (timer_from > 0) {
-            if (timer_from >= solver.max_iters) bis_fatal("block CG: timer_from must be below max_iters");
-            solver.tolerance = 0.0;   // never stop early: exactly max_iters iterations
-        }
-        std::unique_ptr<DeviceCRS> dA = block_matrix(&args, dev, n, rp, col, val, "block CG");
-        int64_t info0[8], info1[8];
-        BIS_OK(bis_context_info(dev, info0));
-        Stopwatch w;
-        w.start();
-        solver.setup(std::move(dA), B, X0);
-        double timed_ms = 0.0;
-        int timed_iters = 0;
-        solver.run(timer_from, &timed_ms, &timed_iters);
-        out_dbl[0] = w.check();
-        out_dbl[1] = timed_ms;
-        BIS_OK(bis_context_info(dev, info1));
-        const std::vector<double> fr = solver.true_residuals();
-        for (int j = 0; j < k; ++j) {
-            const std::vector<double> &h = solver.col_history[(size_t)j];
-            for (size_t i = 0; i < h.size() && i < (size_t)(2 * MAX_ITERS); ++i) history[(size_t)j * 2 * MAX_ITERS + i] = h[i];
-            iter_count[j] = solver.col_iters[(size_t)j];
-            converged[j] = solver.col_converged[(size_t)j];
-            final_res[j] = fr[(size_t)j];
-        }
+        solve_block_with(solver, &args, dev, "block CG", n, rp, col, val, k, B, X0, max_iters, tol, timer_from, history,
+                         iter_count, converged, final_res, out_dbl, out_int);
         if (x_star) BIS_OK(bis_vector_download(dev, x_star, solver.X_old, solver.N * k));
-        out_int[0] = info1[3] - info0[3];
-        out_int[1] = solver.N;
-        out_int[2] = solver.iter_count;
-        out_int[3] = timed_iters;
+        return 0;
+    } catch (const std::exception &e) {
+        g_host_err = e.what();
+        return 1;
+    }
+}
+
+// Gauss-Seidel (sgs = 0) or symmetric Gauss-Seidel (sgs != 0) on k right-hand sides with one matrix
+// (methods/block_gs.hpp).  Arguments and outputs as bis_host_solve_block; precond must be none.
+int bis_host_solve_block_gs(bis_context *dev, const char *matrix_name, int n, const int *rp, const int *col,
+                            const double *val, int k, int precond, int sgs, const double *B, const double *X0,
+                            int max_iters, double tol, int timer_from, double *history, int *iter_count, int *converged,
+                            double *final_res, double *x_star, double *out_dbl, int64_t *out_int) {
+    try {
+        const char *what = sgs ? "block SGS" : "block GS";
+        Args args;
+        args.matrix_file_name = matrix_name ? matrix_name : "in-memory";
+        args.method = sgs ? SolverType::SymmetricGaussSeidel : SolverType::GaussSeidel;
+        args.preconditioner = static_cast<PrecondType>(precond);
+        args.quiet = true;
+        if (!B) bis_fatal(std::string(what) + ": B is required");
+        reject_perm_mode(dev, what);
+        BlockGSSolver solver(&args, dev, k, sgs != 0);
+        solve_block_with(solver, &args, dev, what, n, rp, col, val, k, B, X0, max_iters, tol, timer_from, history,
+                         iter_count, converged, final_res, out_dbl, out_int);
+        if (x_star) BIS_OK(bis_vector_download(dev, x_star, solver.X, solver.N * k));
         return 0;
     } catch (const std::exception &e) {
         g_host_err = e.what();

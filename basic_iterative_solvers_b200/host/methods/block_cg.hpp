@@ -17,46 +17,21 @@
 // slots: [S_B_RR, +k) (r,r) of the newest residual; two banks of (r,z) swapped like the vectors; (Ap,p)
 enum BlockSlot : int { S_B_RR = 32, S_B_RZ_A = 48, S_B_RZ_B = 64, S_B_PAP = 80 };
 
-class BlockCGSolver : public Solver {
+// What the block solvers whose iteration starts with bis_block_cg_status and ends with the k (r,r) slots at S_B_RR share
+// (block CG, block Gauss-Seidel): the device state, the host mirror of the per-column stop decisions, and the loop.
+class BlockSolver : public Solver {
   public:
     int k = 0;
-    double *X_new = nullptr, *X_old = nullptr, *P_new = nullptr, *P_old = nullptr;
-    double *R_new = nullptr, *R_old = nullptr, *Z_new = nullptr, *Z_old = nullptr;
-    double *AP = nullptr, *B = nullptr, *D = nullptr, *state = nullptr;
-    int s_rz = S_B_RZ_A, s_rz_new = S_B_RZ_B;
-    // host mirror of the per-column stop decisions
+    double *state = nullptr;   // [3k] device stop state (bis_block_cg_status)
     std::vector<double> threshold;
     std::vector<int> col_iters;
     std::vector<char> col_active, col_converged;
     std::vector<std::vector<double>> col_history;
 
-    BlockCGSolver(const Args *cli_args, Interface *device, int k_) : Solver(cli_args, device), k(k_) {
-        if (k < 1 || k > BIS_BLOCK_MAX_K) bis_fatal("block CG: k outside [1, BIS_BLOCK_MAX_K]");
-        if (preconditioner != PrecondType::None && preconditioner != PrecondType::Jacobi)
-            bis_fatal("block CG: preconditioner " + to_string(preconditioner) + " not supported (none or jacobi)");
-    }
+    BlockSolver(const Args *cli_args, Interface *device, int k_) : Solver(cli_args, device), k(k_) {}
 
-    // n rows; B_host / X0_host: n x k row-major host arrays (X0 NULL: INIT_X_VAL everywhere)
-    void setup(std::unique_ptr<DeviceCRS> A, const double *B_host, const double *X0_host) {
-        dA = std::move(A);
-        N = dA->n_rows;
-        N_global = dA->n_rows_global;
-        const int64_t nk = N * k;
-        for (double **p : {&X_new, &X_old, &P_new, &P_old, &R_new, &R_old, &Z_new, &Z_old, &AP, &B}) *p = dev_new(dev, nk);
-        state = dev_new(dev, 3 * k);
-        BIS_OK(bis_vector_upload(dev, B, B_host, nk));
-        if (X0_host) BIS_OK(bis_vector_upload(dev, X_old, X0_host, nk));
-        else init_vector(dev, X_old, INIT_X_VAL, nk);
-        init_vector(dev, X_new, 0.0, nk);
-        if (preconditioner == PrecondType::Jacobi) {
-            D = dev_new(dev, N);
-            BIS_OK(bis_matrix_extract_diagonal(dev, dA->handle, D, nullptr));
-        }
-        // cg.hpp:100-120 per column: R = B - A X0, Z = M^-1 R, P = Z, (r,z), (r,r)
-        BIS_OK(bis_spmm(dev, dA->handle, k, X_old, AP));
-        BIS_OK(bis_block_residual(dev, static_cast<int>(preconditioner), N, k, AP, B, D, R_old, Z_old, P_old, s_rz, S_B_RR));
-        std::vector<double> rr(k);
-        BIS_OK(bis_scalar_get(dev, S_B_RR, k, rr.data()));
+    // rr: (r_j, r_j) of the initial residuals; state must be allocated
+    void init_columns(const double *rr) {
         threshold.assign(k, 0.0);
         col_iters.assign(k, 0);
         col_active.assign(k, 1);
@@ -71,25 +46,6 @@ class BlockCGSolver : public Solver {
             st[k + j] = 1.0;
         }
         BIS_OK(bis_vector_upload(dev, state, st.data(), 3 * k));
-    }
-
-    void iterate(Timers *) override {
-        graphed(exchange_count & 1, [&] {
-            const int pc = static_cast<int>(preconditioner);
-            BIS_OK(bis_block_cg_status(dev, k, S_B_RR, max_iters, state));
-            BIS_OK(bis_spmm(dev, dA->handle, k, P_old, AP));
-            BIS_OK(bis_block_dot_to_slots(dev, N, k, AP, P_old, S_B_PAP, state));
-            BIS_OK(bis_block_cg_update(dev, pc, N, k, R_new, R_old, AP, Z_new, D, s_rz, S_B_PAP, S_B_RR, s_rz_new, state));
-            BIS_OK(bis_block_cg_direction_x(dev, N, k, P_new, Z_new, P_old, X_new, X_old, s_rz_new, s_rz, S_B_PAP, state));
-        });
-    }
-    void exchange() override {
-        ++exchange_count;
-        std::swap(P_old, P_new);
-        std::swap(Z_old, Z_new);
-        std::swap(R_old, R_new);
-        std::swap(X_old, X_new);
-        std::swap(s_rz, s_rz_new);
     }
     int n_active() const {
         int a = 0;
@@ -149,6 +105,63 @@ class BlockCGSolver : public Solver {
             if (timed_iters) *timed_iters = iter_count + (ahead ? 1 : 0) - first_timed;
         }
         BIS_OK(bis_context_synchronize(dev));
+    }
+};
+
+class BlockCGSolver : public BlockSolver {
+  public:
+    double *X_new = nullptr, *X_old = nullptr, *P_new = nullptr, *P_old = nullptr;
+    double *R_new = nullptr, *R_old = nullptr, *Z_new = nullptr, *Z_old = nullptr;
+    double *AP = nullptr, *B = nullptr, *D = nullptr;
+    int s_rz = S_B_RZ_A, s_rz_new = S_B_RZ_B;
+
+    BlockCGSolver(const Args *cli_args, Interface *device, int k_) : BlockSolver(cli_args, device, k_) {
+        if (k < 1 || k > BIS_BLOCK_MAX_K) bis_fatal("block CG: k outside [1, BIS_BLOCK_MAX_K]");
+        if (preconditioner != PrecondType::None && preconditioner != PrecondType::Jacobi)
+            bis_fatal("block CG: preconditioner " + to_string(preconditioner) + " not supported (none or jacobi)");
+    }
+
+    // n rows; B_host / X0_host: n x k row-major host arrays (X0 NULL: INIT_X_VAL everywhere)
+    void setup(std::unique_ptr<DeviceCRS> A, const double *B_host, const double *X0_host) {
+        dA = std::move(A);
+        N = dA->n_rows;
+        N_global = dA->n_rows_global;
+        const int64_t nk = N * k;
+        for (double **p : {&X_new, &X_old, &P_new, &P_old, &R_new, &R_old, &Z_new, &Z_old, &AP, &B}) *p = dev_new(dev, nk);
+        state = dev_new(dev, 3 * k);
+        BIS_OK(bis_vector_upload(dev, B, B_host, nk));
+        if (X0_host) BIS_OK(bis_vector_upload(dev, X_old, X0_host, nk));
+        else init_vector(dev, X_old, INIT_X_VAL, nk);
+        init_vector(dev, X_new, 0.0, nk);
+        if (preconditioner == PrecondType::Jacobi) {
+            D = dev_new(dev, N);
+            BIS_OK(bis_matrix_extract_diagonal(dev, dA->handle, D, nullptr));
+        }
+        // cg.hpp:100-120 per column: R = B - A X0, Z = M^-1 R, P = Z, (r,z), (r,r)
+        BIS_OK(bis_spmm(dev, dA->handle, k, X_old, AP));
+        BIS_OK(bis_block_residual(dev, static_cast<int>(preconditioner), N, k, AP, B, D, R_old, Z_old, P_old, s_rz, S_B_RR));
+        std::vector<double> rr(k);
+        BIS_OK(bis_scalar_get(dev, S_B_RR, k, rr.data()));
+        init_columns(rr.data());
+    }
+
+    void iterate(Timers *) override {
+        graphed(exchange_count & 1, [&] {
+            const int pc = static_cast<int>(preconditioner);
+            BIS_OK(bis_block_cg_status(dev, k, S_B_RR, max_iters, state));
+            BIS_OK(bis_spmm(dev, dA->handle, k, P_old, AP));
+            BIS_OK(bis_block_dot_to_slots(dev, N, k, AP, P_old, S_B_PAP, state));
+            BIS_OK(bis_block_cg_update(dev, pc, N, k, R_new, R_old, AP, Z_new, D, s_rz, S_B_PAP, S_B_RR, s_rz_new, state));
+            BIS_OK(bis_block_cg_direction_x(dev, N, k, P_new, Z_new, P_old, X_new, X_old, s_rz_new, s_rz, S_B_PAP, state));
+        });
+    }
+    void exchange() override {
+        ++exchange_count;
+        std::swap(P_old, P_new);
+        std::swap(Z_old, Z_new);
+        std::swap(R_old, R_new);
+        std::swap(X_old, X_new);
+        std::swap(s_rz, s_rz_new);
     }
     // ||b_j - A x*_j|| of every column (x* = X_old); R_new / Z_new are scratch here
     std::vector<double> true_residuals() {

@@ -503,6 +503,28 @@ int bis_block_cg_direction_x(bis_context *ctx, int64_t n, int k, double *P_new,
 int bis_block_cg_status(bis_context *ctx, int k, int slot_rr0, int max_iters,
                         double *state /* [dev] */);
 
+/* Gauss-Seidel sweeps on k columns.
+ * Y = B - T X per column: bis_spmv_sub on each column (Y[i,j] = B[i,j] - s_ij,
+ * s_ij the storage-order sum of bis_spmm).  Checks and profile family as
+ * bis_spmm; NVTX range "spmm_sub". */
+int bis_spmm_sub(bis_context *ctx, const bis_matrix *T, int k, const double *X,
+                 const double *B, double *Y);
+/* X[:, j] = (D + L_strict)^-1 B[:, j] for every column j with active[j] != 0
+ * (all columns if active == NULL), rows ascending as bis_sptrsv, every column
+ * bit-identical to bis_sptrsv on it.  X may alias B.  Columns that are not
+ * active have none of their X entries written.  Works on factors without CRS
+ * arrays (factor_keep_crs = 0); ignores trsv_variant (always the dataflow
+ * schedule).  Two working arrays of n x k doubles are allocated on first use
+ * for the largest k seen (that first call must not be recorded into a graph)
+ * and freed with the factor.  Counted in the "sptrsv" profile family, NVTX
+ * ranges "block-sptrsv" / "block-backwards-sptrsv". */
+int bis_block_sptrsv(bis_context *ctx, const bis_matrix *L_strict, int k, double *X,
+                     const double *D, const double *B,
+                     const double *active /* [dev] k flags, or NULL */);
+/* The same with an upper factor, rows descending as bis_bsptrsv. */
+int bis_block_bsptrsv(bis_context *ctx, const bis_matrix *U_strict, int k, double *X,
+                      const double *D, const double *B, const double *active);
+
 /* Block GMRES (restart length m <= BIS_BLOCK_GMRES_MAX_M): column j runs the
  * arithmetic of the single-RHS GMRES on b_j.
  *
